@@ -483,9 +483,11 @@ def don_leg(dev, peaks_tf32, skip_cpu):
     return leg
 
 
-def run_ours(steps, warmup, n_gpus, skip_cpu=False, legs="all"):
+def run_ours(steps, warmup, n_gpus, skip_cpu=False, legs="all", dump_dir=None):
+    """dump_dir: write the last row of each array the last timed launch returned (rank 0's chains) as <name>.npy there."""
     import statistics
 
+    import numpy as np
     import torch
     import torch.distributed as dist
     from vihmc import engine, samplers
@@ -546,8 +548,16 @@ def run_ours(steps, warmup, n_gpus, skip_cpu=False, legs="all"):
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
             times.append(float(t.item()))
             acc_rate = float(res.accepted.float().mean())
+            if dump_dir is not None and rep == REPS - 1:
+                last_step = {"samples": res.samples[-1], "logp": res.logp[-1], "hamiltonians": res.hamiltonians[-1],
+                             "accepted": res.accepted[-1].float(), "step_sizes": res.step_sizes}
+                last_step = {k: v.cpu().numpy() for k, v in last_step.items()}
             del res
     ms = statistics.median(times)
+    if dump_dir is not None and rank == 0:
+        os.makedirs(dump_dir, exist_ok=True)
+        for name, arr in last_step.items():
+            np.save(os.path.join(dump_dir, f"{name}.npy"), arr)
     evals = world * CHAINS_PER_GPU * steps * (L_STEPS + 1)
     value = evals / (ms * 1e-3)
 
@@ -656,13 +666,20 @@ def main():
     ap.add_argument("--mode", default="intra", choices=["intra", "procs"], help="--impl reference-cfg3 only")
     ap.add_argument("--legs", default="all", choices=["all", "main", "ess", "configs"], help="profiling runs: restrict the extra legs")
     ap.add_argument("--skip-cpu-baseline", action="store_true", help="profiling runs only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last row of each array the last timed launch returned -- samples, logp, hamiltonians, accepted, "
+                         "step_sizes (float32, one .npy each) -- to DIR, to compare two builds output for output")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs is not None and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours only")
     if a.impl == "reference":
         line = run_reference(a.steps, a.warmup, a.gpus)
     elif a.impl == "reference-cfg3":
         line = run_reference_don(a.mode, a.steps)
     else:
-        line = run_ours(a.steps, a.warmup, a.gpus, a.skip_cpu_baseline, a.legs)
+        line = run_ours(a.steps, a.warmup, a.gpus, a.skip_cpu_baseline, a.legs, a.dump_outputs)
     if line is not None:
         if _REAL_STDOUT_FD is not None:
             os.write(_REAL_STDOUT_FD, (json.dumps(line) + "\n").encode())

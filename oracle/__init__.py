@@ -13,14 +13,14 @@ closures.py             torch-CPU restatement of the reference's log-posterior
 hamiltorch_restated.py  restatement of the third-party sampler the reference
                         calls (hamiltorch, unpinned git HEAD, absent here).
 philox_ref.py           numpy Philox4x32-10 + uniform/normal transforms.
-ref_loader.py           imports the REAL reference closures from
-                        /root/reference (build container only).
+ref_loader.py           imports the REAL reference closures from a checkout in
+                        oracle/_ref/ or VIHMC_REFERENCE_ROOT (not in this repository).
 make_golden.py          writes tests/golden/* from the real reference closures.
 
 Parity status
 -------------
 * log-posterior value + gradient: PINNED against the reference's own closures
-  (tests/golden/*.npz were produced by importing /root/reference).
+  (tests/golden/*.npz were produced by importing the original project).
 * sampler arithmetic (hamiltorch): PARITY UNPINNED -- the package is not on
   disk and not pinned by the reference; the restatement is the spec.
 """

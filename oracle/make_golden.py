@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY -- generate tests/golden/* from the REAL reference closures.
 
-Run in the build container (needs /root/reference):
+Needs a checkout of the original VI-HMC project in oracle/_ref/ (or VIHMC_REFERENCE_ROOT=<checkout>):
 
     python oracle/make_golden.py
 

@@ -1,11 +1,12 @@
 """TEST INFRASTRUCTURE ONLY -- loader for the REAL reference closures.
 
-Imports the reference's own ``define_model_log_prob`` factories from
-``/root/reference`` so that golden vectors can be produced from reference code
-rather than from a restatement.  This only works in the build container
-(``/root/reference`` does not exist on the GPU box), so it is used by
-``oracle/make_golden.py`` and by the ``not gpu`` test that re-validates the
-restatement when the reference tree is present.
+Imports the reference's own ``define_model_log_prob`` factories from a checkout
+of the original VI-HMC project so that golden vectors can be produced from
+reference code rather than from a restatement.  The checkout is looked for in
+``oracle/_ref/`` (ignored by git) or wherever ``VIHMC_REFERENCE_ROOT`` points.
+The reference is not part of this repository: ``oracle/make_golden.py`` needs
+it, and the tests compare with its stored outputs (tests/golden/) and re-run it
+live only when it is present.
 
 Obstacles handled here (SURVEY.md section 8(c) "Gotchas"):
   * ``matplotlib`` and ``hamiltorch`` are absent  -> stubbed in ``sys.modules``;
@@ -27,7 +28,7 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("VIHMC_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("VIHMC_REFERENCE_ROOT") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 _LOCAL_MODULES = ("config", "config_splitting", "config_sens", "util", "utils", "my_make_func", "model", "metrics", "bayesian_model",
                   "layers", "layers.BBB", "layers.BBB.BBBLinear", "layers.BBB.BBBConv", "layers.BBB_LRT", "layers.BBB_LRT.BBBLinear",
@@ -78,7 +79,8 @@ def load_script(rel_dir: str, script: str, alias: str):
     can be loaded afterwards.  Returns the module; its ``cfg`` attribute is the script's own config.
     """
     if not reference_available():
-        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT}: put a checkout of the original VI-HMC project there "
+                           "or point VIHMC_REFERENCE_ROOT at one")
     _install_stubs()
     directory = os.path.join(REFERENCE_ROOT, rel_dir)
     saved = {name: sys.modules.pop(name) for name in _LOCAL_MODULES if name in sys.modules}

@@ -1,11 +1,11 @@
 """TEST INFRASTRUCTURE ONLY -- closures with the SHAPE of the reference's ``log_prob_func``.
 
 ``vihmc.closure.spec_from_closure`` recovers a specification from what a reference closure captured
-(free-variable names and the functional-model object behind ``fmodel``).  ``/root/reference`` does not exist on
-the GPU box, so the ``-m gpu`` drop-in tests need closures that capture the same names without importing it.
-The factories below build them on the oracle's restated forward functions; ``tests/test_closure_dropin.py``
-checks (in the build container, where the reference IS present) that the real closures and these yield
-identical recovered specifications, which is what licenses their use on the GPU box.
+(free-variable names and the functional-model object behind ``fmodel``).  The original project is not part of
+this repository, so the tests need closures that capture the same names without importing it.  The factories
+below build them on the oracle's restated forward functions; ``tests/test_closure_dropin.py`` checks that they
+reproduce, bit for bit, the log-posteriors and gradients the original closures gave (tests/golden/), and, when a
+checkout of the original is present, that both yield identical recovered specifications.
 
 Captured names mirrored (reference file:line)
     BNN       x, y, fmodel, dist_list, params_flattened_list, params_shape_list, model, model_loss, tau_out,
@@ -14,6 +14,8 @@ Captured names mirrored (reference file:line)
                                                     Neural_network/VI_HMC/my_make_func.py:24-43
     DeepONet  tr_data, fmodel, dist_list, model_loss, tau_out, prior_scale, predict, nll_loss
                                                     Operator_network/VI_HMC/main_VI_HMC_burgers.py:67-180
+    NUTS      tr_data, fmodel, dist_list, params_flattened_list, model_loss, tau_out, nll_loss
+                                                    Operator_network/HMC/NUTS_DeepOnets.py:120-160
     object    depth_branch, depth_trunk, act, impose_bc, model, learned_mus, learned_sigmas, sampled_weights,
               sensitive_ind                         Operator_network/VI_HMC/my_make_func.py:14-31
     globals   cfg.load_prior, cfg.sample_data, cfg.p main_VI_HMC.py:87,104; main_VI_HMC_burgers.py:76,100,127-137 (from random import sample :14)
@@ -163,5 +165,31 @@ def deeponet_closure(model, model_loss, tr_data, tau_list, tau_out, predict=Fals
         else:
             raise NotImplementedError()
         return ((ll + l_prior / prior_scale), output) if predict else (ll + l_prior / prior_scale)
+
+    return log_prob_func
+
+
+def deeponet_nuts_closure(model, model_loss, tr_data, params_flattened_list, params_shape_list, tau_list, tau_out,
+                          activation="tanh"):
+    """Shape of Operator_network/HMC/NUTS_DeepOnets.py:120-160: one prior per parameter tensor, built as Normal(0, tau * 0.5)
+    (:132, where every other driver takes tau ** 0.5) and walked by the per-tensor slice loop (:144-150)."""
+    f_deeponet = FunctionalDeepONet(depth_branch=model.depth_branch, depth_trunk=model.depth_trunk, activation=activation, model=model)
+    fmodel = f_deeponet.functional_model
+    dist_list = [torch.distributions.Normal(torch.zeros_like(t), t * 0.5) for t in tau_list]
+    nll_loss = torch.nn.GaussianNLLLoss(reduction='sum')
+
+    def log_prob_func(params, *args):
+        l_prior = torch.zeros_like(params[0], requires_grad=True)
+        i_prev = 0
+        for index, shape, dist in zip(params_flattened_list, params_shape_list, dist_list):
+            l_prior = dist.log_prob(params[i_prev:index + i_prev]).sum() + l_prior
+            i_prev += index
+        x1, x2, y = tr_data
+        output = fmodel(x1, x2, parameters=params).squeeze(1)
+        if model_loss == 'NLL':
+            ll = - nll_loss(output, y, tau_out * torch.ones_like(output))
+        else:
+            raise NotImplementedError()
+        return ll + l_prior
 
     return log_prob_func

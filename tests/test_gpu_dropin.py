@@ -158,9 +158,9 @@ def test_subsampling_closure_through_the_shim():
 
 
 # ------------------------------------------------------------------------------------------------
-# the reference's own driver, unmodified, on the GPU (needs the reference tree: VIHMC_REFERENCE_ROOT or /root/reference --
-# its sources may not travel with this repository, so on a box without it the test is skipped; the CPU twin of this test,
-# tests/test_closure_dropin.py, runs in the build container with the oracle standing in for the engine)
+# the reference's own driver, unmodified, on the GPU (needs a checkout of the original project in oracle/_ref/ or VIHMC_REFERENCE_ROOT --
+# its sources are not part of this repository, so without it the test is skipped; the CPU twin of this test,
+# tests/test_closure_dropin.py, runs with the oracle standing in for the engine)
 # ------------------------------------------------------------------------------------------------
 def test_real_reference_driver_main_vi_hmc_on_the_gpu(tmp_path):
     import importlib
@@ -170,7 +170,7 @@ def test_real_reference_driver_main_vi_hmc_on_the_gpu(tmp_path):
     from oracle import ref_loader
 
     if not ref_loader.reference_available():
-        pytest.skip("reference tree not present (set VIHMC_REFERENCE_ROOT)")
+        pytest.skip("original project not present (oracle/_ref/ or VIHMC_REFERENCE_ROOT)")
     saved_mods = {k: sys.modules.pop(k, None) for k in ("hamiltorch", "hamiltorch.samplers", "hamiltorch.util")}
     hamiltorch = importlib.import_module("hamiltorch")
     sys.modules["hamiltorch.util"] = hamiltorch.util

@@ -71,11 +71,11 @@ def test_split_closures_sum_to_full():
 
 
 def test_reference_still_agrees_when_present():
-    """When /root/reference is mounted (build container), re-run one real reference closure live."""
+    """When a checkout of the original project is present (oracle/ref_loader.py), re-run one real reference closure live."""
     from oracle import ref_loader
 
     if not ref_loader.reference_available():
-        pytest.skip("reference tree not mounted (GPU box)")
+        pytest.skip("original project not present (oracle/_ref/ or VIHMC_REFERENCE_ROOT)")
     import os
     import tempfile
 

@@ -1,5 +1,6 @@
-import sys
-sys.path[:0]=['/root/repo','/root/repo/vi-hmc_b200','/root/repo/tests']
+import os, sys
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path[:0] = [ROOT, os.path.join(ROOT, "vi-hmc_b200"), os.path.join(ROOT, "tests")]
 import numpy as np, torch
 import cases
 from vihmc import engine
