@@ -139,6 +139,12 @@ typedef struct vihmc_sampler_io {
   const float* vi_sigma;          /* [D] variational standard deviations */
   float* vi_params;               /* [num_samples, C, D] out (optional): the redrawn weight vectors, what the hook appends to vi_params */
   const float* inject_vi_normals; /* [num_samples, C, D] replaces the Philox N(0,1) draws of the redraw */
+  /* Diagonal mass matrix (hamiltorch's 1-D inv_mass), shared by all chains.  With m = inv_mass, every product separately
+   * rounded: momentum p_i = z_i * sqrt(1 / m_i), kinetic energy 0.5 sum_i p_i (m_i p_i), drift q_i += ((eps m_i) p_i); the
+   * kick is unchanged.  Injected momenta are used as p verbatim (inject already-scaled draws).  Entries must be finite and
+   * > 0: the library cannot check device data without a synchronisation, so this is the caller's contract.  Dense and
+   * per-chain mass matrices are not supported.  m = 1 reproduces the identity run bit for bit. */
+  const float* inv_mass;          /* [d] diagonal inverse mass (hamiltorch inv_mass); NULL = identity */
 } vihmc_sampler_io;
 
 VIHMC_API const char* vihmc_version(void);
@@ -190,6 +196,9 @@ VIHMC_API int vihmc_sample(const vihmc_problem* probs, int32_t n_problems, const
 /* p[C,d] ~ N(0,1): Philox4x32-10, key = seed, counter = (global chain, iteration, d/4 block, stream 0). */
 VIHMC_API int vihmc_momentum_philox(uint64_t seed, int64_t iteration, int64_t chain0, int64_t C, int64_t d, float* p,
                           void* stream);
+/* The same draws scaled for a diagonal mass: p[c,i] = z[c,i] * sqrt(1 / inv_mass[i]) (inv_mass: device [d], finite, > 0). */
+VIHMC_API int vihmc_momentum_philox_mass(uint64_t seed, int64_t iteration, int64_t chain0, int64_t C, int64_t d,
+                               const float* inv_mass, float* p, void* stream);
 /* u[C] ~ U(0,1): counter stream 1. */
 VIHMC_API int vihmc_uniform_philox(uint64_t seed, int64_t iteration, int64_t chain0, int64_t C, float* u, void* stream);
 /* W[C,D] = mu + sigma * N(0,1) (my_make_func.py:45-46 sample_weights), counter stream 2. */
@@ -210,6 +219,14 @@ VIHMC_API int64_t vihmc_ke_partials(int64_t d);
 VIHMC_API int vihmc_kinetic_energy(const float* p, int64_t C, int64_t d, float* ke, float* ke_scratch, void* stream);
 VIHMC_API int vihmc_leapfrog_update(float* q, float* p, const float* g, float eps, const float* eps_per_chain, float kick,
                           float drift, int64_t C, int64_t d, float* ke, float* ke_scratch, void* stream);
+/* Diagonal-mass forms (inv_mass: device [d], finite, > 0, shared by all chains):
+ *   ke[c] = 0.5 sum_i p[c,i] (inv_mass[i] p[c,i]);
+ *   p += kick*eps_c*g ; q += ((drift*eps_c) inv_mass) p ; ke as above. */
+VIHMC_API int vihmc_kinetic_energy_mass(const float* p, const float* inv_mass, int64_t C, int64_t d, float* ke, float* ke_scratch,
+                              void* stream);
+VIHMC_API int vihmc_leapfrog_update_mass(float* q, float* p, const float* g, const float* inv_mass, float eps,
+                               const float* eps_per_chain, float kick, float drift, int64_t C, int64_t d, float* ke,
+                               float* ke_scratch, void* stream);
 /*
  * Metropolis test + state select: accept_c = isfinite(H0_c,H1_c) && min(0, H0_c - H1_c) >= log(u_c);
  * q_cur[c] = accept ? q_prop[c] : q_fallback[c]; on accept q_fallback[c] = q_prop[c]; when `store`
@@ -327,8 +344,8 @@ VIHMC_API int vihmc_debug_xgemm(const float* A, int64_t lda, const float* B, int
                       int32_t N, int32_t K, int32_t batch, void* workspace, size_t workspace_bytes, void* stream);
 
 /*
- * Host-buffer convenience entry (everything is a HOST pointer, including those inside prob): allocates
- * device memory, copies in, runs vihmc_mlp_sample or vihmc_sample, copies samples/diagnostics out.
+ * Host-buffer convenience entry (everything is a HOST pointer, including those inside prob and io, e.g. io->inv_mass[d]):
+ * allocates device memory, copies in, runs vihmc_mlp_sample or vihmc_sample, copies samples/diagnostics out.
  */
 VIHMC_API int vihmc_sample_host(const vihmc_problem* probs_host, int32_t n_problems, const vihmc_sampler_cfg* cfg,
                       int64_t C, const float* q0_host, float* samples_host, const vihmc_sampler_io* io_host);

@@ -48,13 +48,14 @@ int dense_gemm(const float* A, long long a_bs, long long a_sm, long long a_sk, c
                long long b_sn, float* C, long long c_bs, long long ldc, int M, int N, int K, int batch, int use_tc, float* scratch,
                cudaStream_t);
 int row_partials(long long d);
-int launch_momentum(unsigned long long, long long, long long, long long, long long, float*, cudaStream_t);
+int launch_momentum(unsigned long long, long long, long long, long long, long long, const float*, float*, cudaStream_t);
 int launch_uniform(unsigned long long, long long, long long, long long, float*, cudaStream_t);
 int launch_vi_redraw(unsigned long long, long long, long long, long long, long long, const float*, const float*, float*, cudaStream_t);
 int launch_scatter(const float*, const long long*, const float*, float*, long long, long long, long long, cudaStream_t);
 int launch_gather(const long long*, const float*, float*, long long, long long, long long, cudaStream_t);
-int launch_update(float*, float*, const float*, float, const float*, float, float, long long, long long, float*, cudaStream_t);
-int launch_kinetic(const float*, long long, long long, float*, cudaStream_t);
+int launch_update(float*, float*, const float*, float, const float*, float, float, long long, long long, const float*, float*,
+                  cudaStream_t);
+int launch_kinetic(const float*, long long, long long, const float*, float*, cudaStream_t);
 int launch_sum_partials(const float*, int, long long, float*, cudaStream_t);
 int launch_mh_accept(const float*, const float*, const float*, const float*, float*, float*, float*, int, unsigned char*,
                      const float*, float*, float*, long long, long long, cudaStream_t);
@@ -226,7 +227,7 @@ using namespace vihmc;
 // =============================================================================================
 extern "C" {
 
-const char* vihmc_version(void) { return "vihmc 0.1.0 (sm_100a)"; }
+const char* vihmc_version(void) { return "vihmc 0.2.0 (sm_100a)"; }
 const char* vihmc_last_error(void) { return g_error; }
 int vihmc_device_check(void) { return device_check(); }
 
@@ -308,6 +309,7 @@ int vihmc_sample(const vihmc_problem* probs, int32_t n_problems, const vihmc_sam
     model_ws = b > model_ws ? b : model_ws;
   }
   const bool redraw = io != nullptr && io->vi_sigma != nullptr;
+  const float* minv = io != nullptr ? io->inv_mass : nullptr;   // diagonal inverse mass [d], or identity
   const long long Dfull = probs[0].D;
   if (redraw)
     for (int m = 0; m < M; ++m)
@@ -382,8 +384,8 @@ int vihmc_sample(const vihmc_problem* probs, int32_t n_problems, const vihmc_sam
     // momentum + its kinetic energy
     if (io != nullptr && io->inject_momenta != nullptr)
       VIHMC_CUDA_OK(cudaMemcpyAsync(p, io->inject_momenta + (size_t)n * cd, cd * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    else if (int rc = launch_momentum(cfg->seed, n, cfg->chain_offset, C, d, p, st)) return rc;
-    if (int rc = launch_kinetic(p, C, d, ke_part, st)) return rc;
+    else if (int rc = launch_momentum(cfg->seed, n, cfg->chain_offset, C, d, minv, p, st)) return rc;
+    if (int rc = launch_kinetic(p, C, d, minv, ke_part, st)) return rc;
     if (int rc = launch_sum_partials(ke_part, np, C, ke, st)) return rc;
     VIHMC_CUDA_OK(cudaMemcpyAsync(q_prop, q_cur, cd * sizeof(float), cudaMemcpyDeviceToDevice, st));
 
@@ -398,13 +400,13 @@ int vihmc_sample(const vihmc_problem* probs, int32_t n_problems, const vihmc_sam
       if (L == 0) {
         VIHMC_CUDA_OK(cudaMemcpyAsync(H1, H0, C * sizeof(float), cudaMemcpyDeviceToDevice, st));
       } else {
-        if (int rc = launch_update(q_prop, p, g, cfg->step_size, eps, 0.5f, 1.0f, C, d, nullptr, st)) return rc;
+        if (int rc = launch_update(q_prop, p, g, cfg->step_size, eps, 0.5f, 1.0f, C, d, minv, nullptr, st)) return rc;
         for (int s = 1; s <= L; ++s) {
           if (int rc = model_logp_grad(&probs[0], C, q_prop, logp, g, mws, model_ws, st)) return rc;
-          if (int rc = launch_update(q_prop, p, g, cfg->step_size, eps, 1.0f, s < L ? 1.0f : 0.0f, C, d, nullptr, st)) return rc;
+          if (int rc = launch_update(q_prop, p, g, cfg->step_size, eps, 1.0f, s < L ? 1.0f : 0.0f, C, d, minv, nullptr, st)) return rc;
         }
         // hamiltorch: ret_momenta[-1] - 0.5 * step_size * p_grad  (separate rounding, kept)
-        if (int rc = launch_update(q_prop, p, g, cfg->step_size, eps, -0.5f, 0.0f, C, d, ke_part, st)) return rc;
+        if (int rc = launch_update(q_prop, p, g, cfg->step_size, eps, -0.5f, 0.0f, C, d, minv, ke_part, st)) return rc;
         if (int rc = launch_sum_partials(ke_part, np, C, ke, st)) return rc;
         hamiltonian_kernel<<<cb, 128, 0, st>>>(logp, ke, C, H1);
       }
@@ -419,15 +421,15 @@ int vihmc_sample(const vihmc_problem* probs, int32_t n_problems, const vihmc_sam
       for (int s = 0; s < L; ++s) {
         for (int m = 0; m < M; ++m) {
           if (int rc = model_logp_grad(&probs[m], C, q_prop, logp_part, g, mws, model_ws, st)) return rc;
-          if (int rc = launch_update(q_prop, p, g, cfg->step_size, eps, 0.5f, m < M - 1 ? frac : 0.0f, C, d, nullptr, st)) return rc;
+          if (int rc = launch_update(q_prop, p, g, cfg->step_size, eps, 0.5f, m < M - 1 ? frac : 0.0f, C, d, minv, nullptr, st)) return rc;
         }
         for (int m = M - 1; m >= 0; --m) {
           if (int rc = model_logp_grad(&probs[m], C, q_prop, logp_part, g, mws, model_ws, st)) return rc;
-          if (int rc = launch_update(q_prop, p, g, cfg->step_size, eps, 0.5f, m > 0 ? frac : 0.0f, C, d, nullptr, st)) return rc;
+          if (int rc = launch_update(q_prop, p, g, cfg->step_size, eps, 0.5f, m > 0 ? frac : 0.0f, C, d, minv, nullptr, st)) return rc;
         }
       }
       if (int rc = total_logp(q_prop)) return rc;
-      if (int rc = launch_kinetic(p, C, d, ke_part, st)) return rc;
+      if (int rc = launch_kinetic(p, C, d, minv, ke_part, st)) return rc;
       if (int rc = launch_sum_partials(ke_part, np, C, ke, st)) return rc;
       hamiltonian_kernel<<<cb, 128, 0, st>>>(logp, ke, C, H1);
     }
@@ -457,13 +459,25 @@ int vihmc_sample(const vihmc_problem* probs, int32_t n_problems, const vihmc_sam
 
 // ---- building blocks -------------------------------------------------------------------------
 int vihmc_momentum_philox(uint64_t seed, int64_t iteration, int64_t chain0, int64_t C, int64_t d, float* p, void* stream) {
-  return launch_momentum(seed, iteration, chain0, C, d, p, static_cast<cudaStream_t>(stream));
+  return launch_momentum(seed, iteration, chain0, C, d, nullptr, p, static_cast<cudaStream_t>(stream));
 }
-int vihmc_kinetic_energy(const float* p, int64_t C, int64_t d, float* ke, float* ke_scratch, void* stream) {
+int vihmc_momentum_philox_mass(uint64_t seed, int64_t iteration, int64_t chain0, int64_t C, int64_t d, const float* inv_mass, float* p,
+                               void* stream) {
+  if (inv_mass == nullptr) return fail(VIHMC_ERR_INVALID, "momentum_philox_mass: inv_mass is NULL");
+  return launch_momentum(seed, iteration, chain0, C, d, inv_mass, p, static_cast<cudaStream_t>(stream));
+}
+static int kinetic_energy(const float* p, const float* inv_mass, int64_t C, int64_t d, float* ke, float* ke_scratch, void* stream) {
   if (ke == nullptr) return fail(VIHMC_ERR_INVALID, "kinetic_energy: ke is NULL");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (int rc = launch_kinetic(p, C, d, ke_scratch, st)) return rc;
+  if (int rc = launch_kinetic(p, C, d, inv_mass, ke_scratch, st)) return rc;
   return launch_sum_partials(ke_scratch, row_partials(d), C, ke, st);
+}
+int vihmc_kinetic_energy(const float* p, int64_t C, int64_t d, float* ke, float* ke_scratch, void* stream) {
+  return kinetic_energy(p, nullptr, C, d, ke, ke_scratch, stream);
+}
+int vihmc_kinetic_energy_mass(const float* p, const float* inv_mass, int64_t C, int64_t d, float* ke, float* ke_scratch, void* stream) {
+  if (inv_mass == nullptr) return fail(VIHMC_ERR_INVALID, "kinetic_energy_mass: inv_mass is NULL");
+  return kinetic_energy(p, inv_mass, C, d, ke, ke_scratch, stream);
 }
 int vihmc_uniform_philox(uint64_t seed, int64_t iteration, int64_t chain0, int64_t C, float* u, void* stream) {
   return launch_uniform(seed, iteration, chain0, C, u, static_cast<cudaStream_t>(stream));
@@ -481,13 +495,22 @@ int vihmc_gather_vi(const int64_t* sens_ind, const float* grad_W, float* grad_q,
   return launch_gather(reinterpret_cast<const long long*>(sens_ind), grad_W, grad_q, C, D, d, static_cast<cudaStream_t>(stream));
 }
 int64_t vihmc_ke_partials(int64_t d) { return row_partials(d); }
-int vihmc_leapfrog_update(float* q, float* p, const float* g, float eps, const float* eps_per_chain, float kick, float drift,
-                          int64_t C, int64_t d, float* ke, float* ke_scratch, void* stream) {
+static int leapfrog_update(float* q, float* p, const float* g, const float* inv_mass, float eps, const float* eps_per_chain, float kick,
+                           float drift, int64_t C, int64_t d, float* ke, float* ke_scratch, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (ke != nullptr && ke_scratch == nullptr) return fail(VIHMC_ERR_INVALID, "leapfrog_update: ke needs ke_scratch");
-  if (int rc = launch_update(q, p, g, eps, eps_per_chain, kick, drift, C, d, ke ? ke_scratch : nullptr, st)) return rc;
+  if (int rc = launch_update(q, p, g, eps, eps_per_chain, kick, drift, C, d, inv_mass, ke ? ke_scratch : nullptr, st)) return rc;
   if (ke != nullptr) return launch_sum_partials(ke_scratch, row_partials(d), C, ke, st);
   return VIHMC_OK;
+}
+int vihmc_leapfrog_update(float* q, float* p, const float* g, float eps, const float* eps_per_chain, float kick, float drift,
+                          int64_t C, int64_t d, float* ke, float* ke_scratch, void* stream) {
+  return leapfrog_update(q, p, g, nullptr, eps, eps_per_chain, kick, drift, C, d, ke, ke_scratch, stream);
+}
+int vihmc_leapfrog_update_mass(float* q, float* p, const float* g, const float* inv_mass, float eps, const float* eps_per_chain,
+                               float kick, float drift, int64_t C, int64_t d, float* ke, float* ke_scratch, void* stream) {
+  if (inv_mass == nullptr) return fail(VIHMC_ERR_INVALID, "leapfrog_update_mass: inv_mass is NULL");
+  return leapfrog_update(q, p, g, inv_mass, eps, eps_per_chain, kick, drift, C, d, ke, ke_scratch, stream);
 }
 int vihmc_mh_accept(const float* H0, const float* H1, const float* u, const float* q_prop, float* q_cur, float* q_fallback,
                     float* stored_row, int32_t store, uint8_t* accepted, const float* logp_prop, float* logp_fallback,
@@ -533,6 +556,7 @@ int vihmc_sample_host(const vihmc_problem* probs_host, int32_t n_problems, const
     if (io_host->step_sizes && arena.alloc((size_t)C, &io.step_sizes)) return VIHMC_ERR_CUDA;
     if (int rc = arena.upload(io_host->inject_momenta, io_host->inject_momenta ? S * cd : 0, &io.inject_momenta)) return rc;
     if (int rc = arena.upload(io_host->inject_uniforms, io_host->inject_uniforms ? S * C : 0, &io.inject_uniforms)) return rc;
+    if (int rc = arena.upload(io_host->inv_mass, io_host->inv_mass ? (size_t)d : 0, &io.inv_mass)) return rc;
   }
   int rc;
   if (n_problems == 1 && cfg->integrator == VIHMC_INTEGRATOR_LEAPFROG && mlp_small_supported(&dev[0])) {

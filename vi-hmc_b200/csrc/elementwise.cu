@@ -8,6 +8,12 @@
 //
 // All kernels stream [C,d] row-major fp32 once: algorithmic traffic is 20 B/coordinate for the
 // update (read q,p,g; write q,p), 4 B for a momentum draw, 12 B for a VI redraw.
+//
+// Diagonal mass (hamiltorch's 1-D inv_mass m[d], shared by all chains): the MASS instantiations of the
+// momentum, kinetic and update kernels draw p = z * sqrt(1/m), weight the kinetic energy 0.5 sum p (m p)
+// and drift q += ((drift eps) m) p, each product separately rounded.  m is one [d] vector read by scalar
+// __ldg: every chain reads the same entries, so it is served from L1/L2 and adds no HBM traffic per chain.
+// The identity instantiations (MASS = false) are the unchanged kernels.
 #include "common.cuh"
 
 namespace vihmc {
@@ -23,15 +29,26 @@ static inline int grid_for(long long work_items, int per_block) {
 }
 
 // ---------------------------------------------------------------------------------------------
+// sqrt(fl(1 / m)), both correctly rounded: the momentum scale of hamiltorch's Normal(0, (1 / inv_mass) ** 0.5)
+__device__ __forceinline__ float mass_scale(float m) { return __fsqrt_rn(__fdiv_rn(1.0f, m)); }
+
+template <bool MASS>
 __global__ void __launch_bounds__(kThreads) momentum_philox_kernel(unsigned long long seed, unsigned int iteration,
                                                                    long long chain0, long long C, long long d,
-                                                                   float* __restrict__ p) {
+                                                                   const float* __restrict__ inv_mass, float* __restrict__ p) {
   const long long blocks_per_row = (d + 3) / 4;
   const long long total = C * blocks_per_row;
   const bool vec_ok = (d % 4) == 0;
   for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
     const long long c = t / blocks_per_row, j = t % blocks_per_row;
-    const float4 z = philox_normal4(seed, (unsigned long long)(chain0 + c), iteration, (uint32_t)j, STREAM_MOMENTUM);
+    float4 z = philox_normal4(seed, (unsigned long long)(chain0 + c), iteration, (uint32_t)j, STREAM_MOMENTUM);
+    if constexpr (MASS) {
+      const long long i = 4 * j;
+      z.x = __fmul_rn(z.x, mass_scale(__ldg(inv_mass + i)));
+      if (i + 1 < d) z.y = __fmul_rn(z.y, mass_scale(__ldg(inv_mass + i + 1)));
+      if (i + 2 < d) z.z = __fmul_rn(z.z, mass_scale(__ldg(inv_mass + i + 2)));
+      if (i + 3 < d) z.w = __fmul_rn(z.w, mass_scale(__ldg(inv_mass + i + 3)));
+    }
     float* dst = p + c * d + 4 * j;
     if (vec_ok) {
       *reinterpret_cast<float4*>(dst) = z;
@@ -104,10 +121,15 @@ __device__ __forceinline__ int align_phase(const float* p) { return (int)((reint
 constexpr int kUpdVec = 4;                 // float4 per thread per iteration
 constexpr int kUpdSlab = kThreads * kUpdVec * 4;  // coordinates per CTA
 
+// MASS: q += fl(fl(drift eps) m_i) p and ke += p fl(m_i p).  m is indexed by the coordinate, so its 16-byte phase differs from
+// that of q[c*d + i] for odd d; it is therefore NOT part of the phase test below (most chains would fall to the scalar path) and
+// is read by four scalar __ldg inside the float4 loop instead.
+template <bool MASS>
 __global__ void __launch_bounds__(kThreads) leapfrog_update_kernel(float* __restrict__ q, float* __restrict__ p,
                                                                    const float* __restrict__ g, float eps,
                                                                    const float* __restrict__ eps_pc, float kick, float drift,
-                                                                   long long d, float* __restrict__ ke_part, int n_part) {
+                                                                   long long d, const float* __restrict__ inv_mass,
+                                                                   float* __restrict__ ke_part, int n_part) {
   const long long c = blockIdx.y;
   const float e = eps_pc != nullptr ? __ldg(eps_pc + c) : eps;
   const float ck = kick * e, cd = drift * e;
@@ -117,9 +139,15 @@ __global__ void __launch_bounds__(kThreads) leapfrog_update_kernel(float* __rest
   float ke = 0.0f;
   auto scalar = [&](long long i) {
     const float pv = axpy_unfused(ck, g[row + i], p[row + i]);
-    if (drift != 0.0f) q[row + i] = axpy_unfused(cd, pv, q[row + i]);
+    if constexpr (MASS) {
+      const float m = __ldg(inv_mass + i);
+      if (drift != 0.0f) q[row + i] = axpy_unfused(__fmul_rn(cd, m), pv, q[row + i]);
+      ke = fmaf(pv, __fmul_rn(m, pv), ke);
+    } else {
+      if (drift != 0.0f) q[row + i] = axpy_unfused(cd, pv, q[row + i]);
+      ke = fmaf(pv, pv, ke);
+    }
     p[row + i] = pv;
-    ke = fmaf(pv, pv, ke);
   };
   // d is odd for the reference's nets (172 401), so rows start at any alignment: peel to the first 16-byte boundary of
   // this slab, stream float4, finish the tail.  Needs q, p, g to share their alignment phase (else: all scalar).
@@ -134,6 +162,18 @@ __global__ void __launch_bounds__(kThreads) leapfrog_update_kernel(float* __rest
     const float4 gv = *reinterpret_cast<const float4*>(g + row + i);
     pv.x = axpy_unfused(ck, gv.x, pv.x); pv.y = axpy_unfused(ck, gv.y, pv.y);
     pv.z = axpy_unfused(ck, gv.z, pv.z); pv.w = axpy_unfused(ck, gv.w, pv.w);
+    if constexpr (MASS) {
+      const float mx = __ldg(inv_mass + i), my = __ldg(inv_mass + i + 1), mz = __ldg(inv_mass + i + 2), mw = __ldg(inv_mass + i + 3);
+      if (drift != 0.0f) {
+        qv.x = axpy_unfused(__fmul_rn(cd, mx), pv.x, qv.x); qv.y = axpy_unfused(__fmul_rn(cd, my), pv.y, qv.y);
+        qv.z = axpy_unfused(__fmul_rn(cd, mz), pv.z, qv.z); qv.w = axpy_unfused(__fmul_rn(cd, mw), pv.w, qv.w);
+        *reinterpret_cast<float4*>(q + row + i) = qv;
+      }
+      *reinterpret_cast<float4*>(p + row + i) = pv;
+      ke = fmaf(pv.x, __fmul_rn(mx, pv.x), ke); ke = fmaf(pv.y, __fmul_rn(my, pv.y), ke);
+      ke = fmaf(pv.z, __fmul_rn(mz, pv.z), ke); ke = fmaf(pv.w, __fmul_rn(mw, pv.w), ke);
+      continue;
+    }
     if (drift != 0.0f) {
       qv.x = axpy_unfused(cd, pv.x, qv.x); qv.y = axpy_unfused(cd, pv.y, qv.y);
       qv.z = axpy_unfused(cd, pv.z, qv.z); qv.w = axpy_unfused(cd, pv.w, qv.w);
@@ -164,14 +204,19 @@ __global__ void sum_partials_kernel(const float* __restrict__ part, int n_part, 
   out[c] = s;
 }
 
-// kinetic energy of a fresh momentum (no update): same partial layout
-__global__ void __launch_bounds__(kThreads) kinetic_kernel(const float* __restrict__ p, long long d, float* __restrict__ ke_part,
+// kinetic energy of a fresh momentum (no update): same partial layout; MASS: 0.5 sum_i p_i fl(m_i p_i)
+template <bool MASS>
+__global__ void __launch_bounds__(kThreads) kinetic_kernel(const float* __restrict__ p, long long d,
+                                                           const float* __restrict__ inv_mass, float* __restrict__ ke_part,
                                                            int n_part) {
   const long long c = blockIdx.y, row = c * d;
   const long long lo = (long long)blockIdx.x * kUpdSlab;
   const long long hi = lo + kUpdSlab < d ? lo + kUpdSlab : d;
   float ke = 0.0f;
-  for (long long i = lo + threadIdx.x; i < hi; i += kThreads) ke = fmaf(p[row + i], p[row + i], ke);
+  for (long long i = lo + threadIdx.x; i < hi; i += kThreads) {
+    if constexpr (MASS) ke = fmaf(p[row + i], __fmul_rn(__ldg(inv_mass + i), p[row + i]), ke);
+    else ke = fmaf(p[row + i], p[row + i], ke);
+  }
   __shared__ float red[kThreads / 32];
   ke = warp_sum(ke);
   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = ke;
@@ -234,11 +279,15 @@ __global__ void __launch_bounds__(kThreads) mh_accept_kernel(const float* __rest
 // ---------------------------------------------------------------------------------------------
 int row_partials(long long d) { return (int)((d + kUpdSlab - 1) / kUpdSlab); }
 
-int launch_momentum(unsigned long long seed, long long iteration, long long chain0, long long C, long long d, float* p,
-                    cudaStream_t st) {
+// inv_mass: [d] diagonal inverse mass, or nullptr (identity)
+int launch_momentum(unsigned long long seed, long long iteration, long long chain0, long long C, long long d, const float* inv_mass,
+                    float* p, cudaStream_t st) {
   if (C < 1 || d < 1 || p == nullptr) return fail(VIHMC_ERR_INVALID, "momentum_philox: bad arguments");
   const long long items = C * ((d + 3) / 4);
-  momentum_philox_kernel<<<grid_for(items, kThreads), kThreads, 0, st>>>(seed, (unsigned int)iteration, chain0, C, d, p);
+  if (inv_mass != nullptr)
+    momentum_philox_kernel<true><<<grid_for(items, kThreads), kThreads, 0, st>>>(seed, (unsigned int)iteration, chain0, C, d, inv_mass, p);
+  else
+    momentum_philox_kernel<false><<<grid_for(items, kThreads), kThreads, 0, st>>>(seed, (unsigned int)iteration, chain0, C, d, nullptr, p);
   VIHMC_LAUNCH_OK("momentum_philox_kernel");
   return VIHMC_OK;
 }
@@ -282,20 +331,27 @@ int launch_gather(const long long* ind, const float* gW, float* gq, long long C,
 
 // ke_part may be NULL; otherwise [C, row_partials(d)]
 int launch_update(float* q, float* p, const float* g, float eps, const float* eps_pc, float kick, float drift, long long C,
-                  long long d, float* ke_part, cudaStream_t st) {
+                  long long d, const float* inv_mass, float* ke_part, cudaStream_t st) {
   if (C < 1 || d < 1 || !q || !p || !g) return fail(VIHMC_ERR_INVALID, "leapfrog_update: bad arguments");
   if (C > 65535) return fail(VIHMC_ERR_UNSUPPORTED, "leapfrog_update: more than 65535 chains per call");
   const int np = row_partials(d);
-  leapfrog_update_kernel<<<dim3(np, (unsigned)C), kThreads, 0, st>>>(q, p, g, eps, eps_pc, kick, drift, d, ke_part, np);
+  const dim3 grid(np, (unsigned)C);
+  if (inv_mass != nullptr)
+    leapfrog_update_kernel<true><<<grid, kThreads, 0, st>>>(q, p, g, eps, eps_pc, kick, drift, d, inv_mass, ke_part, np);
+  else
+    leapfrog_update_kernel<false><<<grid, kThreads, 0, st>>>(q, p, g, eps, eps_pc, kick, drift, d, nullptr, ke_part, np);
   VIHMC_LAUNCH_OK("leapfrog_update_kernel");
   return VIHMC_OK;
 }
 
-int launch_kinetic(const float* p, long long C, long long d, float* ke_part, cudaStream_t st) {
+int launch_kinetic(const float* p, long long C, long long d, const float* inv_mass, float* ke_part, cudaStream_t st) {
   if (C < 1 || d < 1 || !p || !ke_part) return fail(VIHMC_ERR_INVALID, "kinetic_energy: bad arguments");
   if (C > 65535) return fail(VIHMC_ERR_UNSUPPORTED, "kinetic_energy: more than 65535 chains per call");
   const int np = row_partials(d);
-  kinetic_kernel<<<dim3(np, (unsigned)C), kThreads, 0, st>>>(p, d, ke_part, np);
+  if (inv_mass != nullptr)
+    kinetic_kernel<true><<<dim3(np, (unsigned)C), kThreads, 0, st>>>(p, d, inv_mass, ke_part, np);
+  else
+    kinetic_kernel<false><<<dim3(np, (unsigned)C), kThreads, 0, st>>>(p, d, nullptr, ke_part, np);
   VIHMC_LAUNCH_OK("kinetic_kernel");
   return VIHMC_OK;
 }

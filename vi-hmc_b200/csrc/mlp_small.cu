@@ -194,6 +194,13 @@ int mlp_small_sample(const vihmc_problem* prob, const vihmc_sampler_cfg* cfg, lo
   int W = 0;
   SmallLaunch a{};
   if (int rc = fill_params(prob, P, W, C, true, a.fast)) return rc;
+  if (io != nullptr && io->inv_mass != nullptr) {
+    // diagonal mass: the same variant with the per-coordinate m_i, s_i region appended to each chain's shared memory
+    P.lay = make_layout(W, P.n_hidden, P.in_dim, P.d, a.fast, true);
+    if ((size_t)P.lay.total * sizeof(float) > 227u * 1024u)
+      return fail(VIHMC_ERR_UNSUPPORTED, "mlp_sample: d = %lld with a diagonal mass does not fit one CTA's shared memory", (long long)P.d);
+    a.A.inv_mass = io->inv_mass;
+  }
   pick_geometry(P, C, a);
   a.A.cfg = *cfg; a.A.C = C; a.A.q0 = q0; a.A.samples = samples;
   if (io != nullptr) {

@@ -51,6 +51,7 @@ struct SmallLayout {
   int part, pmeta;   // specialised path v2: per-lane partial gradient sums [2W+9 slots][33] and each coordinate's offset into them
   int perm;          // v2, register-resident coordinates: coordinate index of (lane, round), 64 entries (-1: none)
   int rot;           // v2: hidden->hidden tables in schedule order (column 2m + h of row j holds unit fast2_unit_at(JP, j % JP, m) + JP h)
+  int minv, msq;     // sampler with a diagonal mass only (empty otherwise): inv_mass m_i and sqrt(1 / m_i), dp entries each
   int total;
 };
 
@@ -115,8 +116,9 @@ constexpr bool fast2_row_loads_conflict_free(int W) {   // per step and quarter 
 static_assert(fast2_schedule_is_a_permutation(5) && fast2_schedule_is_a_permutation(8), "spare-row schedule must visit every unit once");
 static_assert(fast2_row_loads_conflict_free(10) && fast2_row_loads_conflict_free(16), "row shifts must keep the activation-quad loads conflict-free");
 
-// W = padded hidden width the kernel is compiled for; fast = layout of the specialised 1-W-W-1 tanh path
-__host__ __device__ constexpr SmallLayout make_layout(int W, int n_hidden, int in_dim, long long d, int fast = 0) {
+// W = padded hidden width the kernel is compiled for; fast = layout of the specialised 1-W-W-1 tanh path; mass = the sampler's
+// diagonal-mass region (appended last, so no other offset moves)
+__host__ __device__ constexpr SmallLayout make_layout(int W, int n_hidden, int in_dim, long long d, int fast = 0, bool mass = false) {
   SmallLayout L{};
   const int WSW = round_up(W, 4);
   int off = 0;
@@ -159,6 +161,8 @@ __host__ __device__ constexpr SmallLayout make_layout(int W, int n_hidden, int i
   L.part = off; off += fast ? (2 * W + 9) * 33 + 3 : 0;
   L.perm = off; off += fast ? 64 : 0;
   L.rot = fast >= 2 ? 1 : 0;
+  L.minv = off; off += mass ? L.dp : 0;
+  L.msq = off; off += mass ? L.dp : 0;
   L.total = off;
   return L;
 }
@@ -377,8 +381,10 @@ __device__ __forceinline__ float stage_chunk(float* sm, const SmallParams& P, in
 
 // One-time per-chain setup: zero the weight tables, load frozen weights, decode coordinates, load
 // the prior and q (scattered into the tables).  Returns this thread's target when N fits one chunk.
-template <int W, int NW>
-__device__ float chain_init(float* sm, const SmallParams& P, const float* q_row, int ct, int bar, long long chain = 0) {
+// MASS (sampler with a diagonal mass): also m_i = inv_mass[i] and s_i = sqrt(fl(1 / m_i)), both correctly rounded.
+template <int W, int NW, bool MASS = false>
+__device__ float chain_init(float* sm, const SmallParams& P, const float* q_row, int ct, int bar, long long chain = 0,
+                            const float* inv_mass = nullptr) {
   using C = Cfg<W, NW>;
   const SmallLayout& L = P.lay;
   for (int i = ct; i < L.w_total; i += C::T) sm[i] = 0.0f;                 // padded units and weight-row padding stay zero
@@ -407,6 +413,11 @@ __device__ float chain_init(float* sm, const SmallParams& P, const float* q_row,
     const float sig = P.prior_sigma ? __ldg(P.prior_sigma + i) : P.prior_sigma_scalar;
     sm[L.piv + i] = isinf(sig) ? 0.0f : 1.0f / (sig * sig);
     sm[L.pmu + i] = P.prior_mu ? __ldg(P.prior_mu + i) : 0.0f;
+    if constexpr (MASS) {
+      const float m = __ldg(inv_mass + i);
+      sm[L.minv + i] = m;
+      sm[L.msq + i] = __fsqrt_rn(__fdiv_rn(1.0f, m));
+    }
     const float qv = q_row[i];
     sm[L.q + i] = qv;
     sm[L.qf + i] = qv;
@@ -1175,9 +1186,12 @@ struct SampleArgs {
   const float* vi_sigma;   // per-sample VI redraw (vihmc_sampler_io): [D] standard deviations, or null
   float* vi_params;        // [num_samples, C, D] out, or null
   const float* inj_vi;     // [num_samples, C, D] injected normals, or null
+  const float* inv_mass;   // [d] diagonal inverse mass (the MASS instantiation), or null
 };
 
-template <int W, int NW, int FAST>
+// MASS: diagonal mass m = A.inv_mass (hamiltorch's 1-D inv_mass).  p = fl(z s_i), ke = 0.5 sum p fl(m_i p), drift
+// q += fl(fl(eps m_i) p); with MASS = false the code is exactly the identity-mass kernel.
+template <int W, int NW, int FAST, bool MASS>
 __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHMC_SMALL_MINBLOCKS) mlp_small_sample_kernel(SmallParams P, SampleArgs A) {
   extern __shared__ __align__(16) float smem[];
   constexpr int T = Cfg<W, NW>::T;
@@ -1190,7 +1204,7 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
   const int d = (int)P.d;
   const long long C = A.C;
   const float* q0 = A.q0 + chain * d;
-  const float yv0 = chain_init<W, NW>(sm, P, q0, ct, bar, chain);
+  const float yv0 = chain_init<W, NW, MASS>(sm, P, q0, ct, bar, chain, A.inv_mass);
   FastRegs F;
   if constexpr (FAST != 0) fast_setup<W>(sm, ct, yv0, F);
   if constexpr (FAST >= 2) fast2_setup<W>(sm, P, ct);
@@ -1201,6 +1215,7 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
   int r_pm[NR], r_wpos[NR], r_wposT[NR], r_idx[NR];
   const int nq_used = ((int)P.N + 3) / 4;
   float r_pmu[NR], r_piv[NR], r_q[NR], r_p[NR];
+  float r_m[NR];   // MASS: the lane's inverse masses (s_i is read from shared memory by the once-per-iteration momentum draw)
   bool r_ok[NR];
   if constexpr (FAST == 3) {
     const int* pmv = reinterpret_cast<const int*>(sm + L.pmeta);
@@ -1217,6 +1232,7 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
       r_wposT[r] = r_ok[r] ? wtv[i] : -1;
       r_pmu[r] = r_ok[r] ? sm[L.pmu + i] : 0.0f;
       r_piv[r] = r_ok[r] ? sm[L.piv + i] : 0.0f;
+      if constexpr (MASS) r_m[r] = r_ok[r] ? sm[L.minv + i] : 0.0f;
       r_q[r] = r_p[r] = 0.0f;
     }
   }
@@ -1279,9 +1295,10 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
     if (A.inj_p != nullptr) {
       const float* src = A.inj_p + ((long long)n * C + chain) * d;
       for (int i = ct; i < d; i += T) {
-        const float pv = src[i];
+        const float pv = src[i];   // injected momenta are used as p verbatim (already scaled for the mass)
         sm[L.p + i] = pv;
-        ke = fmaf(pv, pv, ke);
+        if constexpr (MASS) ke = fmaf(pv, __fmul_rn(sm[L.minv + i], pv), ke);
+        else ke = fmaf(pv, pv, ke);
       }
     } else {
       for (int jb = ct; 4 * jb < d; jb += T) {
@@ -1290,8 +1307,15 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
 #pragma unroll
         for (int t = 0; t < 4; ++t)
           if (4 * jb + t < d) {
-            sm[L.p + 4 * jb + t] = zz[t];
-            ke = fmaf(zz[t], zz[t], ke);
+            if constexpr (MASS) {
+              const int i = 4 * jb + t;
+              const float pv = __fmul_rn(zz[t], sm[L.msq + i]);
+              sm[L.p + i] = pv;
+              ke = fmaf(pv, __fmul_rn(sm[L.minv + i], pv), ke);
+            } else {
+              sm[L.p + 4 * jb + t] = zz[t];
+              ke = fmaf(zz[t], zz[t], ke);
+            }
           }
       }
     }
@@ -1323,8 +1347,14 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
           const float gi = r_ok[r] ? fmaf(-dq * iv, P.inv_prior_scale, gl[r]) : 0.0f;
           const float pk = axpy_unfused(kick, gi, r_p[r]);
           const float pv = last ? __fsub_rn(pk, __fmul_rn(half_eps, gi)) : pk;
-          ke_lane = fmaf(pv, pv, ke_lane);            // read only after the last evaluation
-          const float qv = axpy_unfused(eps, pv, r_q[r]);
+          float qv;
+          if constexpr (MASS) {
+            ke_lane = fmaf(pv, __fmul_rn(r_m[r], pv), ke_lane);   // read only after the last evaluation
+            qv = axpy_unfused(__fmul_rn(eps, r_m[r]), pv, r_q[r]);
+          } else {
+            ke_lane = fmaf(pv, pv, ke_lane);            // read only after the last evaluation
+            qv = axpy_unfused(eps, pv, r_q[r]);
+          }
           r_q[r] = last ? r_q[r] : qv;
           r_p[r] = pv;
           if (!last && r_ok[r]) sm[r_wpos[r]] = qv;
@@ -1347,9 +1377,10 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
         if (last) {
           // hamiltorch: p += eps*g inside the loop, then ret_momenta[-1] - 0.5*eps*g (separately rounded)
           pv = __fsub_rn(pv, __fmul_rn(half_eps, gi));
-          ke_lane = fmaf(pv, pv, ke_lane);
+          if constexpr (MASS) ke_lane = fmaf(pv, __fmul_rn(sm[L.minv + i], pv), ke_lane);
+          else ke_lane = fmaf(pv, pv, ke_lane);
         } else {
-          const float qv = axpy_unfused(eps, pv, qv0);
+          const float qv = axpy_unfused(MASS ? __fmul_rn(eps, sm[L.minv + i]) : eps, pv, qv0);
           sm[L.q + i] = qv;
           sm[wposv[i]] = qv;
           const int wt = wposTv[i];
@@ -1454,7 +1485,7 @@ static int set_smem(K kernel, size_t bytes) {
   return VIHMC_OK;
 }
 
-template <int W, int NW, int FAST>
+template <int W, int NW, int FAST, bool MASS = false>
 static int launch_small_wn(SmallOp op, const SmallParams& P, const SmallLaunch& a, cudaStream_t st) {
   const int threads = a.chains_per_block * 32 * NW;
   if (op == kOpLogpGrad) {
@@ -1473,7 +1504,7 @@ static int launch_small_wn(SmallOp op, const SmallParams& P, const SmallLaunch& 
     k<<<a.blocks, threads, a.smem, st>>>(P, a.C, a.q, a.out);
     VIHMC_LAUNCH_OK("mlp_small_predict_kernel");
   } else {
-    auto k = mlp_small_sample_kernel<W, NW, FAST>;
+    auto k = mlp_small_sample_kernel<W, NW, FAST, MASS>;
     if (int rc = set_smem(k, a.smem)) return rc;
     k<<<a.blocks, threads, a.smem, st>>>(P, a.A);
     VIHMC_LAUNCH_OK("mlp_small_sample_kernel");
@@ -1481,15 +1512,22 @@ static int launch_small_wn(SmallOp op, const SmallParams& P, const SmallLaunch& 
   return VIHMC_OK;
 }
 
+// the sampler with a diagonal mass takes the MASS instantiation of the same variant (only the sample kernel has one)
+template <int W, int NW, int FAST>
+static int launch_small_wm(SmallOp op, const SmallParams& P, const SmallLaunch& a, cudaStream_t st) {
+  if (op == kOpSample && a.A.inv_mass != nullptr) return launch_small_wn<W, NW, FAST, true>(op, P, a, st);
+  return launch_small_wn<W, NW, FAST, false>(op, P, a, st);
+}
+
 template <int W>
 static int launch_small_w(SmallOp op, const SmallParams& P, const SmallLaunch& a, cudaStream_t st) {
-  if (a.warps_per_chain == 2) return launch_small_wn<W, 2, 0>(op, P, a, st);
+  if (a.warps_per_chain == 2) return launch_small_wm<W, 2, 0>(op, P, a, st);
   if constexpr (W <= 16) {   // version 2 keeps 2 W quads in registers: widths above 16 stay on version 1
-    if (a.fast == 2 && op == kOpSample && P.d <= 32 * kRegRounds) return launch_small_wn<W, 1, 3>(op, P, a, st);
-    if (a.fast == 2) return launch_small_wn<W, 1, 2>(op, P, a, st);
+    if (a.fast == 2 && op == kOpSample && P.d <= 32 * kRegRounds) return launch_small_wm<W, 1, 3>(op, P, a, st);
+    if (a.fast == 2) return launch_small_wm<W, 1, 2>(op, P, a, st);
   }
-  if (a.fast) return launch_small_wn<W, 1, 1>(op, P, a, st);
-  return launch_small_wn<W, 1, 0>(op, P, a, st);
+  if (a.fast) return launch_small_wm<W, 1, 1>(op, P, a, st);
+  return launch_small_wm<W, 1, 0>(op, P, a, st);
 }
 
 }  // namespace vihmc

@@ -42,6 +42,7 @@ class SamplerIO(C.Structure):
         ("accepted", C.c_void_p), ("hamiltonians", C.c_void_p), ("logp", C.c_void_p), ("step_sizes", C.c_void_p),
         ("inject_momenta", C.c_void_p), ("inject_uniforms", C.c_void_p),
         ("vi_sigma", C.c_void_p), ("vi_params", C.c_void_p), ("inject_vi_normals", C.c_void_p),
+        ("inv_mass", C.c_void_p),
     ]
 
 
@@ -88,6 +89,9 @@ SYMBOLS = {
     "vihmc_vi_epoch_end": (C.c_int, [C.POINTER(ViCfg), _I64, _V, _I32, _F, _V, _V, _V, _V, _SZ, _V]),
     "vihmc_debug_umma": (C.c_int, [_V, _V] + [C.c_uint32] * 7 + [_V, _V]),
     "vihmc_kinetic_energy": (C.c_int, [_V, _I64, _I64, _V, _V, _V]),
+    "vihmc_momentum_philox_mass": (C.c_int, [_U64, _I64, _I64, _I64, _I64, _V, _V, _V]),
+    "vihmc_kinetic_energy_mass": (C.c_int, [_V, _V, _I64, _I64, _V, _V, _V]),
+    "vihmc_leapfrog_update_mass": (C.c_int, [_V, _V, _V, _V, _F, _V, _F, _F, _I64, _I64, _V, _V, _V]),
     "vihmc_debug_tanh": (C.c_int, [_I32, _V, _V, _I64, _V]),
     "vihmc_debug_xgemm_workspace_bytes": (_SZ, [_I32, _I32, _I32]),
     "vihmc_debug_xgemm": (C.c_int, [_V, _I64, _V, _I64, _V, _I64, _I32, _I32, _I32, _I32, _V, _SZ, _V]),

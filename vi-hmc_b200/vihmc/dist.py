@@ -83,7 +83,8 @@ def sample_sharded(specs, q0_all: torch.Tensor, total_chains: int, burn_in_draws
 
     q0_all: [total_chains, d] start points (every rank passes the same tensor; each takes its rows).
     burn_in_draws: stored rows to drop before the diagnostics (the caller-side `params_hmc[cfg.burn:]`).
-    Returns {'samples','logp','accepted' (rank 0: full; else None), 'rhat' (all ranks), 'local'}."""
+    Returns {'samples','logp','accepted' (rank 0: full; else None), 'rhat' (all ranks), 'local'}.
+    ``sampler_kw`` goes to ``engine.run_sampler`` as it is, including ``inv_mass`` (one [d] diagonal for every chain of every rank)."""
     from . import engine
 
     chain0, n_local = shard_chains(total_chains)
@@ -116,7 +117,8 @@ def shard_spec_rows(spec, rank: Optional[int] = None, world_size: Optional[int] 
 
 
 def sample_data_sharded(spec_local, q0: torch.Tensor, num_samples: int, num_steps: int, step_size: float, burn: int = 0,
-                        seed: int = 0, hamiltorch_fallback_rule: bool = True, use_graphs: bool = True) -> Dict[str, torch.Tensor]:
+                        seed: int = 0, hamiltorch_fallback_rule: bool = True, use_graphs: bool = True,
+                        inv_mass: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
     """HMC where every rank holds ALL chains and a row shard of the data (spec_local = shard_spec_rows(spec)).
 
     One exchange step per gradient evaluation: ONE all_reduce(SUM) of a [C, d + 1] buffer (gradients, log-posterior behind them);
@@ -129,7 +131,11 @@ def sample_data_sharded(spec_local, q0: torch.Tensor, num_samples: int, num_step
     back, H1) -- gradient kernels, the packed all-reduce and the update kernels -- are each captured once into a CUDA graph (NCCL
     collectives are capturable) and replayed: with 8 GPUs a step is well under a millisecond of ~40 short launches, and the
     replay removes the launch gaps.  Same kernels, same order, same results as the eager loop
-    (tests/test_gpu_deeponet.py::test_data_sharded_sampler_equals_general_sampler compares the two bit for bit)."""
+    (tests/test_gpu_deeponet.py::test_data_sharded_sampler_equals_general_sampler compares the two bit for bit).
+
+    ``inv_mass``: diagonal inverse mass [d] as in ``engine.run_sampler``.  The captured graphs read it by address, so the graph
+    cache is keyed on the device tensor's ``data_ptr()`` and holds a reference to it: pass the same device tensor again to replay,
+    a different one re-captures."""
     from . import engine
 
     rank, w = world()
@@ -148,17 +154,25 @@ def sample_data_sharded(spec_local, q0: torch.Tensor, num_samples: int, num_step
     accepted = torch.empty((num_samples, C), dtype=torch.uint8, device=dev)
     ham = torch.empty((num_samples, C, 2), dtype=torch.float32, device=dev)
     q_cur, q_fb = q0d.clone(), q0d.clone()
+    m = None
+    if inv_mass is not None:
+        m = inv_mass if isinstance(inv_mass, torch.Tensor) else torch.as_tensor(inv_mass)
+        m = m.to(device=dev, dtype=torch.float32).contiguous()
+        if m.shape != (d,):
+            raise ValueError(f"inv_mass must be a 1-D tensor of length d={d}")
 
     # Work buffers and graphs are cached on the prepared problem, keyed by what the captured launches depend on: a second call
     # with the same chains / step size (the timed call after a warm-up, the next block of iterations) replays without re-capturing.
     cache = prep.__dict__.setdefault("_data_sharded_cache", {})
-    key = (C, d, float(step_size), w, bool(use_graphs))
+    key = (C, d, float(step_size), w, bool(use_graphs), None if m is None else m.data_ptr())
     st = cache.get(key)
     if st is None:
         st = cache[key] = {"q": torch.empty_like(q0d), "p": torch.empty_like(q0d),
+                           "inv_mass": m,   # the graphs read it by address: keep it alive as long as they are
+
                            # ONE collective per evaluation: the [C] log-posteriors ride behind the [C, d] gradients in the same buffer
                            "packed": torch.empty((C, d + 1), dtype=torch.float32, device=dev) if w > 1 else None, "graphs": None}
-    q, p, packed = st["q"], st["p"], st["packed"]
+    q, p, packed, m = st["q"], st["p"], st["packed"], st["inv_mass"]
 
     def grad(qq):
         lp, g = engine.logp_grad(prep, qq)
@@ -172,19 +186,19 @@ def sample_data_sharded(spec_local, q0: torch.Tensor, num_samples: int, num_step
 
     def step_first():
         lp, g = grad(q)
-        ke0 = engine.leapfrog_update(q, p, g, step_size, 0.0, 0.0, want_ke=True)     # kinetic energy of the fresh momentum
+        ke0 = engine.leapfrog_update(q, p, g, step_size, 0.0, 0.0, want_ke=True, inv_mass=m)   # kinetic energy of the fresh momentum
         h0 = ke0 - lp
-        engine.leapfrog_update(q, p, g, step_size, 0.5, 1.0)
+        engine.leapfrog_update(q, p, g, step_size, 0.5, 1.0, inv_mass=m)
         return h0
 
     def step_mid():
         lp, g = grad(q)
-        engine.leapfrog_update(q, p, g, step_size, 1.0, 1.0)
+        engine.leapfrog_update(q, p, g, step_size, 1.0, 1.0, inv_mass=m)
 
     def step_last():
         lp, g = grad(q)
-        engine.leapfrog_update(q, p, g, step_size, 1.0, 0.0)
-        ke1 = engine.leapfrog_update(q, p, g, step_size, -0.5, 0.0, want_ke=True)
+        engine.leapfrog_update(q, p, g, step_size, 1.0, 0.0, inv_mass=m)
+        ke1 = engine.leapfrog_update(q, p, g, step_size, -0.5, 0.0, want_ke=True, inv_mass=m)
         return ke1 - lp
 
     # a trajectory of L steps: first, L - 1 middle evaluations, last (L + 1 gradient evaluations)
@@ -217,7 +231,7 @@ def sample_data_sharded(spec_local, q0: torch.Tensor, num_samples: int, num_step
     for n in range(num_samples):
         if hamiltorch_fallback_rule and n == burn + 1:
             q_fb.copy_(q0d)
-        p.copy_(engine.momentum_philox(seed, n, 0, C, d, device=dev))
+        p.copy_(engine.momentum_philox(seed, n, 0, C, d, device=dev, inv_mass=m))
         q.copy_(q_cur)
         h0 = run("first", step_first)
         for s in range(1, num_steps):

@@ -193,8 +193,12 @@ def run_sampler(specs: Sequence, q0: torch.Tensor, num_samples: int, num_steps: 
                 seed: int = 0, chain_offset: int = 0, hamiltorch_fallback_rule: bool = True, diagnostics: bool = True,
                 inject_momenta: Optional[torch.Tensor] = None, inject_uniforms: Optional[torch.Tensor] = None,
                 to_host: bool = True, force_general: bool = False, vi_redraw: bool = False,
-                inject_vi_normals: Optional[torch.Tensor] = None) -> SampleResult:
+                inject_vi_normals: Optional[torch.Tensor] = None, inv_mass: Optional[torch.Tensor] = None) -> SampleResult:
     """Advance C = q0.shape[0] chains.  specs: one LogProbSpec/Prepared (leapfrog) or several (splitting).
+
+    inv_mass: hamiltorch's 1-D ``inv_mass`` [d], a diagonal inverse mass shared by all chains (finite, > 0; validated by
+    ``samplers.sample``): momenta p = z sqrt(1 / m), kinetic energy 0.5 p.(m p), drift q += eps m p.  Injected momenta are used
+    as p verbatim.  None is the identity mass.
 
     vi_redraw: the reference's ``sample_weights`` hook once per iteration (Neural_network/VI_HMC/my_make_func.py:45-50): all D
     frozen weights of every chain are redrawn from N(mu, sigma) (spec.frozen, spec.vi_sigma; Philox stream 2 or
@@ -232,6 +236,10 @@ def run_sampler(specs: Sequence, q0: torch.Tensor, num_samples: int, num_steps: 
     if inj_u is not None:
         assert tuple(inj_u.shape) == (num_samples, Cn), inj_u.shape
         io.inject_uniforms = inj_u.data_ptr()
+    minv = _to_dev(inv_mass, dev)
+    if minv is not None:
+        assert tuple(minv.shape) == (d,), minv.shape
+        io.inv_mass = minv.data_ptr()
     vip = vsig = inj_v = None
     if vi_redraw:
         sp0 = preps[0].spec
@@ -311,13 +319,15 @@ class _TrunkSubset:
 
 def run_sampler_trunk_subsample(spec, q0: torch.Tensor, num_samples: int, num_steps: int, step_size: float, burn: int = 0,
                                 seed: int = 0, chain_offset: int = 0, inject_momenta: Optional[torch.Tensor] = None,
-                                inject_uniforms: Optional[torch.Tensor] = None, to_host: bool = True) -> SampleResult:
+                                inject_uniforms: Optional[torch.Tensor] = None, to_host: bool = True,
+                                inv_mass: Optional[torch.Tensor] = None) -> SampleResult:
     """HMC for a DeepONet closure with cfg.sample_data: EVERY closure call -- the two Hamiltonians and the L + 1 gradients of an
     iteration, L + 3 calls as hamiltorch makes them -- sees a fresh ``random.sample(range(P), p)`` of the trunk points
     (Operator_network/VI_HMC/main_VI_HMC_burgers.py:127-137).  The subsets come from Python's global ``random`` exactly as in the
     reference (seed it for reproducibility); all chains of the call share them.  The iteration is composed on the host from the
     exported building blocks (vihmc_momentum_philox, vihmc_logp_grad on the gathered problem, vihmc_leapfrog_update,
-    vihmc_mh_accept): a DeepONet evaluation is milliseconds of GPU work, so the Python loop only enqueues."""
+    vihmc_mh_accept): a DeepONet evaluation is milliseconds of GPU work, so the Python loop only enqueues.  ``inv_mass``: diagonal
+    inverse mass [d] as in :func:`run_sampler` (the ``_mass`` building blocks)."""
     import random
 
     prep = prepare(spec)
@@ -336,6 +346,7 @@ def run_sampler_trunk_subsample(spec, q0: torch.Tensor, num_samples: int, num_st
     ham = torch.empty((num_samples, Cn, 2), dtype=torch.float32, device=dev)
     fb_burn, fb_post = q.clone(), q.clone()   # param_burn_prev / ret_params[-1] of hamiltorch
     inj_p, inj_u = _to_dev(inject_momenta, dev), _to_dev(inject_uniforms, dev)
+    m = _to_dev(inv_mass, dev)
 
     # the L + 3 subsets of an iteration are drawn on the host in the order the closure calls consume them and uploaded ONCE
     # (pinned, non-blocking); the closures then gather from device-resident index rows, so the loop really only enqueues
@@ -355,20 +366,20 @@ def run_sampler_trunk_subsample(spec, q0: torch.Tensor, num_samples: int, num_st
         except RuntimeError:
             pass
         subsets["dev"], subsets["next"] = host_idx.to(dev, non_blocking=True), 0
-        p = inj_p[n].clone() if inj_p is not None else momentum_philox(seed, n, chain_offset, Cn, d, dev)
+        p = inj_p[n].clone() if inj_p is not None else momentum_philox(seed, n, chain_offset, Cn, d, dev, inv_mass=m)
         u = inj_u[n].contiguous() if inj_u is not None else uniform_philox(seed, n, chain_offset, Cn, dev)
         q_prop = q.clone()
         lp0, _ = closure().logp_grad(q_prop, need_grad=False)
-        ke0 = kinetic_energy(p)
+        ke0 = kinetic_energy(p, inv_mass=m)
         _, g = closure().logp_grad(q_prop)
-        leapfrog_update(q_prop, p, g, step_size, 0.5, 1.0)                 # p += eps/2 g ; q += eps p
+        leapfrog_update(q_prop, p, g, step_size, 0.5, 1.0, inv_mass=m)                 # p += eps/2 g ; q += eps p
         for s_ in range(1, num_steps + 1):
             _, g = closure().logp_grad(q_prop)
             if s_ < num_steps:
-                leapfrog_update(q_prop, p, g, step_size, 1.0, 1.0)         # p += eps g ; q += eps p
+                leapfrog_update(q_prop, p, g, step_size, 1.0, 1.0, inv_mass=m)         # p += eps g ; q += eps p
             else:
-                leapfrog_update(q_prop, p, g, step_size, 1.0, 0.0)         # p += eps g
-        ke1 = leapfrog_update(q_prop, p, g, step_size, -0.5, 0.0, want_ke=True)   # p -= eps/2 g
+                leapfrog_update(q_prop, p, g, step_size, 1.0, 0.0, inv_mass=m)         # p += eps g
+        ke1 = leapfrog_update(q_prop, p, g, step_size, -0.5, 0.0, want_ke=True, inv_mass=m)   # p -= eps/2 g
         lp1, _ = closure().logp_grad(q_prop, need_grad=False)
         H0, H1 = ke0 - lp0, ke1 - lp1
         ham[n, :, 0].copy_(H0)
@@ -385,11 +396,19 @@ def run_sampler_trunk_subsample(spec, q0: torch.Tensor, num_samples: int, num_st
     return res
 
 
-def momentum_philox(seed: int, iteration: int, chain0: int, chains: int, d: int, device=None) -> torch.Tensor:
+def momentum_philox(seed: int, iteration: int, chain0: int, chains: int, d: int, device=None,
+                    inv_mass: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """p [C, d] ~ N(0, 1) (Philox stream 0); with ``inv_mass`` [d] the same draws times sqrt(1 / inv_mass)."""
     dev = _require_cuda(device)
     p = torch.empty((chains, d), dtype=torch.float32, device=dev)
+    m = _to_dev(inv_mass, dev)
     with torch.cuda.device(dev):
-        _lib.check(_lib.load().vihmc_momentum_philox(seed, iteration, chain0, chains, d, p.data_ptr(), _stream(dev)))
+        if m is None:
+            _lib.check(_lib.load().vihmc_momentum_philox(seed, iteration, chain0, chains, d, p.data_ptr(), _stream(dev)))
+        else:
+            assert m.numel() == d, m.shape
+            _lib.check(_lib.load().vihmc_momentum_philox_mass(seed, iteration, chain0, chains, d, m.data_ptr(), p.data_ptr(),
+                                                              _stream(dev)))
     return p
 
 
@@ -426,8 +445,10 @@ def scatter_vi(frozen: torch.Tensor, sens_ind, q: torch.Tensor) -> torch.Tensor:
 
 
 def leapfrog_update(q: torch.Tensor, p: torch.Tensor, g: torch.Tensor, eps: float, kick: float, drift: float,
-                    eps_per_chain: Optional[torch.Tensor] = None, want_ke: bool = False):
-    """In-place fused update on device tensors q,p [C,d]; returns ke[C] if requested."""
+                    eps_per_chain: Optional[torch.Tensor] = None, want_ke: bool = False,
+                    inv_mass: Optional[torch.Tensor] = None):
+    """In-place fused update on device tensors q,p [C,d]; returns ke[C] if requested.  With ``inv_mass`` [d] (a device fp32
+    tensor) the drift is q += ((drift eps) inv_mass) p and ke = 0.5 p.(inv_mass p) (vihmc_leapfrog_update_mass)."""
     dev = _require_cuda(q.device)
     Cn, d = q.shape
     lib = _lib.load()
@@ -436,20 +457,30 @@ def leapfrog_update(q: torch.Tensor, p: torch.Tensor, g: torch.Tensor, eps: floa
         ke = torch.empty(Cn, dtype=torch.float32, device=dev)
         scratch = torch.empty(Cn * int(lib.vihmc_ke_partials(d)), dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
-        _lib.check(lib.vihmc_leapfrog_update(q.data_ptr(), p.data_ptr(), g.data_ptr(), eps, _ptr(eps_per_chain), kick, drift,
-                                             Cn, d, _ptr(ke), _ptr(scratch), _stream(dev)))
+        if inv_mass is None:
+            _lib.check(lib.vihmc_leapfrog_update(q.data_ptr(), p.data_ptr(), g.data_ptr(), eps, _ptr(eps_per_chain), kick, drift,
+                                                 Cn, d, _ptr(ke), _ptr(scratch), _stream(dev)))
+        else:
+            assert inv_mass.is_cuda and inv_mass.dtype == torch.float32 and inv_mass.numel() == d and inv_mass.is_contiguous()
+            _lib.check(lib.vihmc_leapfrog_update_mass(q.data_ptr(), p.data_ptr(), g.data_ptr(), inv_mass.data_ptr(), eps,
+                                                      _ptr(eps_per_chain), kick, drift, Cn, d, _ptr(ke), _ptr(scratch), _stream(dev)))
     return ke
 
 
-def kinetic_energy(p: torch.Tensor) -> torch.Tensor:
-    """ke[c] = 0.5 sum p[c]^2 (vihmc_kinetic_energy)."""
+def kinetic_energy(p: torch.Tensor, inv_mass: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """ke[c] = 0.5 sum p[c]^2 (vihmc_kinetic_energy); with ``inv_mass`` [d] (device fp32) 0.5 sum p[c] (inv_mass p[c])."""
     dev = _require_cuda(p.device)
     Cn, d = p.shape
     lib = _lib.load()
     ke = torch.empty(Cn, dtype=torch.float32, device=dev)
     scratch = torch.empty(Cn * int(lib.vihmc_ke_partials(d)), dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
-        _lib.check(lib.vihmc_kinetic_energy(p.data_ptr(), Cn, d, ke.data_ptr(), scratch.data_ptr(), _stream(dev)))
+        if inv_mass is None:
+            _lib.check(lib.vihmc_kinetic_energy(p.data_ptr(), Cn, d, ke.data_ptr(), scratch.data_ptr(), _stream(dev)))
+        else:
+            assert inv_mass.is_cuda and inv_mass.dtype == torch.float32 and inv_mass.numel() == d and inv_mass.is_contiguous()
+            _lib.check(lib.vihmc_kinetic_energy_mass(p.data_ptr(), inv_mass.data_ptr(), Cn, d, ke.data_ptr(), scratch.data_ptr(),
+                                                     _stream(dev)))
     return ke
 
 

@@ -17,7 +17,8 @@ What changes at this boundary: ``log_prob_func`` is a :class:`vihmc.spec.LogProb
 for ``Integrator.SPLITTING``) -- either built by the factories below, or recovered from one of the reference's own
 closures by ``vihmc.closure.spec_from_closure`` (so the reference's drivers run unmodified through the ``hamiltorch``
 drop-in package) and checked once against that closure at ``params_init``.  New optional keywords: ``num_chains``
-(params_init may also be ``[C, d]``), ``seed``, ``chain_offset``, ``return_result``.  With one chain the
+(params_init may also be ``[C, d]``), ``seed``, ``chain_offset``, ``return_result``.  hamiltorch's ``inv_mass`` is supported
+in its 1-D (diagonal) form.  With one chain the
 return value is hamiltorch's list of ``num_samples - burn`` 1-D tensors (so ``np.save`` writes the same
 ``(S, d)`` array); with C chains it is a ``[S - burn, C, d]`` tensor.
 """
@@ -67,6 +68,25 @@ def _initial_states(spec: LogProbSpec, params_init: torch.Tensor, num_chains: Op
     return q
 
 
+def check_inv_mass(inv_mass, d: int) -> Optional[torch.Tensor]:
+    """hamiltorch's ``inv_mass`` as the engine takes it: None, or a 1-D length-d array of finite, positive entries (a diagonal
+    inverse mass shared by all chains), returned as a CPU fp32 tensor.  Checked on the host so that nothing reaches the GPU
+    with a mass the kernels cannot use; the dense (2-D) and block-list forms are not implemented."""
+    if inv_mass is None:
+        return None
+    if isinstance(inv_mass, (list, tuple)):
+        raise NotImplementedError("inv_mass as a list of blocks is not implemented; pass the diagonal as a 1-D tensor of length d")
+    m = inv_mass.detach().cpu() if isinstance(inv_mass, torch.Tensor) else torch.as_tensor(np.asarray(inv_mass))
+    if m.dim() == 2:
+        raise NotImplementedError("a dense (2-D) inv_mass is not implemented; pass the diagonal as a 1-D tensor of length d")
+    if m.dim() != 1 or m.shape[0] != d:
+        raise ValueError(f"inv_mass must be a 1-D tensor of length d={d}, got shape {tuple(m.shape)}")
+    m = m.to(torch.float32)
+    if not bool(torch.isfinite(m).all()) or not bool((m > 0).all()):
+        raise ValueError("inv_mass entries must be finite and > 0")
+    return m.contiguous()
+
+
 def sample(log_prob_func, params_init, num_samples=10, num_steps_per_sample=10, step_size=0.1, burn=0, jitter=None,
            inv_mass=None, normalizing_const=1., softabs_const=None, explicit_binding_const=100,
            fixed_point_threshold=1e-5, fixed_point_max_iterations=1000, jitter_max_tries=10, sampler=Sampler.HMC,
@@ -80,11 +100,13 @@ def sample(log_prob_func, params_init, num_samples=10, num_steps_per_sample=10, 
     vi_redraw=True runs the reference's per-sample VI redraw -- what a sampler does that calls ``log_prob_func(params, True)`` once
     per sample (main_VI_HMC.py:96-99 -> my_make_func.py:45-50 ``sample_weights``): every frozen weight is redrawn from its
     variational N(mu, sigma) at the start of each iteration; with ``vi_params_uid`` the draws are written to
-    ``vi_params_<uid>.npy`` as the hook does ([num_samples, D] for one chain, [num_samples, C, D] for C chains)."""
+    ``vi_params_<uid>.npy`` as the hook does ([num_samples, D] for one chain, [num_samples, C, D] for C chains).
+
+    inv_mass: hamiltorch's diagonal inverse mass, a 1-D tensor or array of length d with finite, positive entries, shared by
+    all chains (``check_inv_mass``).  ``params_std[grad_ind] ** 2`` from the VI fit is the natural choice for VI-HMC; the
+    step size must then be re-tuned (``Sampler.HMC_NUTS`` does).  Injected momenta are used as given, i.e. already scaled."""
     if sampler == Sampler.RMHMC:
         raise NotImplementedError("RMHMC is not used by the reference and is not on the accelerated path")
-    if inv_mass is not None:
-        raise NotImplementedError("only the identity mass matrix (the reference's setting) is implemented")
     specs = list(log_prob_func) if isinstance(log_prob_func, (list, tuple)) else [log_prob_func]
     closures = {}
     for i, s in enumerate(specs):
@@ -113,6 +135,7 @@ def sample(log_prob_func, params_init, num_samples=10, num_steps_per_sample=10, 
     if nuts and burn == 0:
         raise RuntimeError("burn must be greater than 0 for NUTS.")
     spec0 = specs[0].spec if isinstance(specs[0], engine.Prepared) else specs[0]
+    inv_mass = check_inv_mass(inv_mass, spec0.d)
     single = isinstance(params_init, torch.Tensor) and params_init.dim() == 1 and num_chains in (None, 1)
     q0 = _initial_states(spec0, params_init, num_chains, seed)
     if closures and verify_closures:
@@ -128,7 +151,7 @@ def sample(log_prob_func, params_init, num_samples=10, num_steps_per_sample=10, 
             raise NotImplementedError("trunk sub-sampling (cfg.sample_data) is implemented for plain HMC with one log-posterior")
         res = engine.run_sampler_trunk_subsample(specs[0], q0, num_samples, num_steps_per_sample, float(step_size), burn=burn, seed=seed,
                                                  chain_offset=chain_offset, inject_momenta=inject_momenta,
-                                                 inject_uniforms=inject_uniforms, to_host=True)
+                                                 inject_uniforms=inject_uniforms, to_host=True, inv_mass=inv_mass)
         if verbose or debug:
             print("Acceptance Rate {:.2f}".format(res.acceptance_rate))
         if return_result:
@@ -138,7 +161,7 @@ def sample(log_prob_func, params_init, num_samples=10, num_steps_per_sample=10, 
                              adapt_step_size=nuts, desired_accept_rate=desired_accept_rate, seed=seed,
                              chain_offset=chain_offset, hamiltorch_fallback_rule=hamiltorch_fallback_rule,
                              inject_momenta=inject_momenta, inject_uniforms=inject_uniforms, to_host=True, vi_redraw=vi_redraw,
-                             inject_vi_normals=inject_vi_normals)
+                             inject_vi_normals=inject_vi_normals, inv_mass=inv_mass)
     if vi_redraw and vi_params_uid is not None:
         vp = res.vi_params[:, 0] if single else res.vi_params
         np.save(f"vi_params_{vi_params_uid}.npy", vp.clone().detach().cpu())
@@ -242,7 +265,7 @@ def sample_model(model, x, y, params_init, model_loss='multi_class_linear_output
                  fixed_point_max_iterations=1000, jitter_max_tries=10, sampler=Sampler.HMC, integrator=Integrator.IMPLICIT,
                  metric=Metric.HESSIAN, debug=False, tau_out=1., tau_list=None, store_on_GPU=True,
                  desired_accept_rate=0.8, verbose=False, **engine_kw):
-    """hamiltorch.sample_model as called at Neural_network/HMC/main_regression_hmc.py:124-127."""
+    """hamiltorch.sample_model as called at Neural_network/HMC/main_regression_hmc.py:124-127 (``inv_mass``: as in ``sample``)."""
     numels = [w.nelement() for w in model.parameters()]
     shapes = [w.shape for w in model.parameters()]
     if tau_list is None:
@@ -250,7 +273,7 @@ def sample_model(model, x, y, params_init, model_loss='multi_class_linear_output
     spec = define_model_log_prob_hamiltorch(model, model_loss, x, y, numels, shapes, tau_list, tau_out,
                                             normalizing_const=normalizing_const)
     return sample(spec, params_init, num_samples=num_samples, num_steps_per_sample=num_steps_per_sample,
-                  step_size=step_size, burn=burn, sampler=sampler, integrator=integrator, debug=debug,
+                  step_size=step_size, burn=burn, inv_mass=inv_mass, sampler=sampler, integrator=integrator, debug=debug,
                   desired_accept_rate=desired_accept_rate, verbose=verbose, **engine_kw)
 
 
