@@ -64,8 +64,7 @@ print("VARIANT OK")
 """
 
 
-@pytest.mark.parametrize("env", [{}, {"VIHMC_SMALL_GENERIC": "1"}, {"VIHMC_SMALL_FAST": "1"}, {"VIHMC_SMALL_NW": "2"}],
-                         ids=["default", "generic", "fast1", "nw2"])
+@pytest.mark.parametrize("env", [{}, {"VIHMC_SMALL_GENERIC": "1"}, {"VIHMC_SMALL_FAST": "1"}], ids=["default", "generic", "fast1"])
 def test_persistent_kernel_ones_mass_is_identity_in_every_variant(env):
     """The persistent kernel's variants are chosen by environment knobs read once per process, so each runs in a subprocess.
     default covers fast v2 with register-resident coordinates (d40, d14) and without (d141)."""

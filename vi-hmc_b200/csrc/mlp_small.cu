@@ -29,12 +29,11 @@ bool mlp_small_supported(const vihmc_problem* p) {
   return (size_t)L.total * sizeof(float) <= 200u * 1024u;  // one chain must fit in one CTA's smem
 }
 
-static int warps_per_chain_for(long long C);
 static bool fast_path_enabled();
 static int fast_version();
 
 // allow_fast: the caller's kernel has a specialised variant (log-posterior/gradient and the sampler; not predict)
-static int fill_params(const vihmc_problem* p, SmallParams& P, int& W, long long C, bool allow_fast, int& fast) {
+static int fill_params(const vihmc_problem* p, SmallParams& P, int& W, bool allow_fast, int& fast) {
   if (!mlp_small_supported(p))
     return fail(VIHMC_ERR_UNSUPPORTED, "MLP outside the small-net kernel's range (<=4 hidden layers of width <=32, out_dim 1)");
   if (p->x == nullptr || p->y == nullptr) return fail(VIHMC_ERR_INVALID, "x and y must be device pointers");
@@ -62,8 +61,7 @@ static int fill_params(const vihmc_problem* p, SmallParams& P, int& W, long long
   P.prior_sigma_scalar = p->prior_sigma_scalar; P.prior_log_norm = p->prior_log_norm;
   P.x = p->x; P.y = p->y; P.frozen = p->frozen; P.frozen_cs = p->frozen_chain_stride; P.prior_mu = p->prior_mu; P.prior_sigma = p->prior_sigma;
   P.sens_ind = reinterpret_cast<const long long*>(p->sens_ind);
-  fast = allow_fast && fast_path_enabled() && warps_per_chain_for(C) == 1 && nh == 2 && p->in_a == 1 && p->act == VIHMC_ACT_TANH &&
-         p->N <= (32 / W) * 8;
+  fast = allow_fast && fast_path_enabled() && nh == 2 && p->in_a == 1 && p->act == VIHMC_ACT_TANH && p->N <= (32 / W) * 8;
   if (fast && W <= 16 && p->last_bias) fast = fast_version();
   P.lay = make_layout(W, nh, p->in_a, p->d, fast);
   return VIHMC_OK;
@@ -72,20 +70,6 @@ static int fill_params(const vihmc_problem* p, SmallParams& P, int& W, long long
 int mlp_small_launch_w10(SmallOp, const SmallParams&, const SmallLaunch&, cudaStream_t);
 int mlp_small_launch_w16(SmallOp, const SmallParams&, const SmallLaunch&, cudaStream_t);
 int mlp_small_launch_w32(SmallOp, const SmallParams&, const SmallLaunch&, cudaStream_t);
-
-// Geometry.  Warps per chain: 1.  Splitting a chain over 2 warps (VIHMC_SMALL_NW=2, kept for experiments) doubles
-// the resident warps but measured SLOWER on B200 at 1024 chains (313 M vs 489 M chain-grad-evals/s): the 64-thread
-// named barriers between phases and the halved per-lane ILP cost more than the extra TLP hides.  Chains per CTA: 1 for few chains so the
-// 148 SMs fill evenly, up to 4 warps per CTA for many chains so the 32-CTA/SM limit does not cap residency.
-static int warps_per_chain_for(long long C) {
-  static const int forced = []() {
-    const char* e = getenv("VIHMC_SMALL_NW");
-    return (e != nullptr && (e[0] == '1' || e[0] == '2')) ? e[0] - '0' : 0;
-  }();
-  if (forced) return forced;
-  (void)C;
-  return 1;
-}
 
 // VIHMC_SMALL_GENERIC=1 keeps every problem on the generic evaluation (the A/B baseline of the bit-exactness test)
 static bool fast_path_enabled() {
@@ -105,14 +89,13 @@ static int fast_version() {
   return v;
 }
 
+// Geometry: one warp per chain; 1 chain per CTA for few chains so the 148 SMs fill evenly, up to 4 for many chains so
+// the 32-CTA/SM limit does not cap residency.
 static void pick_geometry(const SmallParams& P, long long C, SmallLaunch& a) {
   const SmallLayout& L = P.lay;
   const size_t per_chain = (size_t)L.total * sizeof(float);
-  const int nw = warps_per_chain_for(C);
-
   int cpb = 1;
-  while (cpb * nw < 4 && C > (long long)148 * 24 * cpb && per_chain * (cpb * 2) <= 200u * 1024u) cpb *= 2;
-  a.warps_per_chain = nw;
+  while (cpb < 4 && C > (long long)148 * 24 * cpb && per_chain * (cpb * 2) <= 200u * 1024u) cpb *= 2;
   a.chains_per_block = cpb;
   a.blocks = (int)((C + cpb - 1) / cpb);
   a.smem = per_chain * cpb;
@@ -130,7 +113,7 @@ int mlp_small_logp_grad(const vihmc_problem* prob, long long C, const float* q, 
   SmallParams P{};
   int W = 0;
   SmallLaunch a{};
-  if (int rc = fill_params(prob, P, W, C, true, a.fast)) return rc;
+  if (int rc = fill_params(prob, P, W, true, a.fast)) return rc;
   pick_geometry(P, C, a);
   a.q = q; a.logp = logp; a.grad = grad;
   return dispatch(W, kOpLogpGrad, P, a, st);
@@ -140,7 +123,7 @@ int mlp_small_predict(const vihmc_problem* prob, long long C, const float* q, fl
   SmallParams P{};
   int W = 0;
   SmallLaunch a{};
-  if (int rc = fill_params(prob, P, W, C, false, a.fast)) return rc;
+  if (int rc = fill_params(prob, P, W, false, a.fast)) return rc;
   pick_geometry(P, C, a);
   a.q = q; a.out = out;
   return dispatch(W, kOpPredict, P, a, st);
@@ -176,11 +159,11 @@ int mlp_small_sensitivity(const vihmc_problem* prob, const float* weights, const
   SmallParams P{};
   int W = 0;
   SmallLaunch a{};
-  if (int rc = fill_params(&p, P, W, 1, false, a.fast)) return rc;
+  if (int rc = fill_params(&p, P, W, false, a.fast)) return rc;
   const size_t need = mlp_small_sensitivity_workspace(&p);
   if (ws == nullptr || ws_bytes < need) return fail(VIHMC_ERR_WORKSPACE, "sensitivity: workspace too small, need %zu bytes", need);
   const int chunks = (int)((P.N + P.lay.NC - 1) / P.lay.NC);
-  a.warps_per_chain = 1; a.chains_per_block = 1; a.blocks = chunks; a.smem = (size_t)P.lay.total * sizeof(float); a.C = 1;
+  a.chains_per_block = 1; a.blocks = chunks; a.smem = (size_t)P.lay.total * sizeof(float); a.C = 1;
   a.q = weights; a.out = static_cast<float*>(ws);
   if (int rc = dispatch(W, kOpSensitivity, P, a, st)) return rc;
   sensitivity_finish_kernel<<<(unsigned)((P.d + 127) / 128), 128, 0, st>>>(a.out, chunks, P.d, P.N, sigma, out);
@@ -193,7 +176,7 @@ int mlp_small_sample(const vihmc_problem* prob, const vihmc_sampler_cfg* cfg, lo
   SmallParams P{};
   int W = 0;
   SmallLaunch a{};
-  if (int rc = fill_params(prob, P, W, C, true, a.fast)) return rc;
+  if (int rc = fill_params(prob, P, W, true, a.fast)) return rc;
   if (io != nullptr && io->inv_mass != nullptr) {
     // diagonal mass: the same variant with the per-coordinate m_i, s_i region appended to each chain's shared memory
     P.lay = make_layout(W, P.n_hidden, P.in_dim, P.d, a.fast, true);

@@ -47,7 +47,7 @@ struct SmallLayout {
   int act_base, xs, h, da, dz, dO, ones, act_total;
   int NC, NCS;
   // per-coordinate state, each dp entries
-  int coord_base, dp, q, p, g, qf, pmu, piv, meta, wpos, wposT, red;
+  int coord_base, dp, q, p, g, qf, pmu, piv, meta, wpos, wposT;
   int part, pmeta;   // specialised path v2: per-lane partial gradient sums [2W+9 slots][33] and each coordinate's offset into them
   int perm;          // v2, register-resident coordinates: coordinate index of (lane, round), 64 entries (-1: none)
   int rot;           // v2: hidden->hidden tables in schedule order (column 2m + h of row j holds unit fast2_unit_at(JP, j % JP, m) + JP h)
@@ -156,7 +156,6 @@ __host__ __device__ constexpr SmallLayout make_layout(int W, int n_hidden, int i
   L.meta = off; off += L.dp;
   L.wpos = off; off += L.dp;
   L.wposT = off; off += L.dp;
-  L.red = off; off += 8;      // cross-warp reduction slots (two warps per chain)
   L.pmeta = off; off += fast ? L.dp : 0;
   L.part = off; off += fast ? (2 * W + 9) * 33 + 3 : 0;
   L.perm = off; off += fast ? 64 : 0;
@@ -327,45 +326,23 @@ __device__ __forceinline__ void dot_rows2(const float* wrow, const float* rows, 
 }
 
 // ------------------------------------------------------------------------------------------------
-// chain-level geometry: NW warps cooperate on one chain (NW = 1: everything is warp-synchronous;
-// NW = 2: twice the warps per SM to hide latency when the chain count is small, 4 points per lane,
-// phases separated by a 64-thread named barrier)
+// chain-level geometry: one warp per chain, so every phase is warp-synchronous (__syncwarp between phases)
 // ------------------------------------------------------------------------------------------------
-template <int W, int NW>
+template <int W>
 struct Cfg {
-  static constexpr int T = 32 * NW;          // threads per chain
+  static constexpr int T = 32;               // threads per chain
   static constexpr int NC = (32 / W) * 8;    // data points per chunk
   static constexpr int NCS = NC + 4;         // activation row stride
-  static constexpr int PPL = 8 / NW;         // data points per lane in unit mode
+  static constexpr int PPL = 8;              // data points per lane in unit mode
   static constexpr int G = NC / PPL;         // point groups
   static constexpr int WSW = (W + 3) / 4 * 4;
   static_assert(G * W <= T, "unit-mode lanes exceed the chain's threads");
 };
 
-template <int NW>
-__device__ __forceinline__ void chain_sync(int bar) {
-  if (NW == 1) __syncwarp();
-  else asm volatile("bar.sync %0, %1;" ::"r"(bar), "n"(32 * NW) : "memory");
-}
-
-// sum over all threads of the chain, same value on every thread (fixed order => reproducible)
-template <int NW>
-__device__ __forceinline__ float chain_sum(float v, float* red, int ct, int bar) {
-  v = warp_sum(v);
-  if (NW == 1) return v;
-  if ((ct & 31) == 0) red[ct >> 5] = v;
-  chain_sync<NW>(bar);
-  float s = 0.0f;
-#pragma unroll
-  for (int w = 0; w < NW; ++w) s += red[w];
-  chain_sync<NW>(bar);
-  return s;
-}
-
 // point-mode staging of one data chunk: x columns, validity row; returns this thread's target
-template <int W, int NW>
+template <int W>
 __device__ __forceinline__ float stage_chunk(float* sm, const SmallParams& P, int ct, int chunk) {
-  using C = Cfg<W, NW>;
+  using C = Cfg<W>;
   const SmallLayout& L = P.lay;
   float* act = sm + L.act_base;
   float yv = 0.0f;
@@ -382,14 +359,14 @@ __device__ __forceinline__ float stage_chunk(float* sm, const SmallParams& P, in
 // One-time per-chain setup: zero the weight tables, load frozen weights, decode coordinates, load
 // the prior and q (scattered into the tables).  Returns this thread's target when N fits one chunk.
 // MASS (sampler with a diagonal mass): also m_i = inv_mass[i] and s_i = sqrt(fl(1 / m_i)), both correctly rounded.
-template <int W, int NW, bool MASS = false>
-__device__ float chain_init(float* sm, const SmallParams& P, const float* q_row, int ct, int bar, long long chain = 0,
+template <int W, bool MASS = false>
+__device__ float chain_init(float* sm, const SmallParams& P, const float* q_row, int ct, long long chain = 0,
                             const float* inv_mass = nullptr) {
-  using C = Cfg<W, NW>;
+  using C = Cfg<W>;
   const SmallLayout& L = P.lay;
   for (int i = ct; i < L.w_total; i += C::T) sm[i] = 0.0f;                 // padded units and weight-row padding stay zero
   for (int i = L.coord_base + ct; i < L.total; i += C::T) sm[i] = 0.0f;
-  chain_sync<NW>(bar);
+  __syncwarp();
   if (P.frozen != nullptr) {
     for (long long f = ct; f < P.D; f += C::T) {
       int wpos, wposT, a, b;
@@ -399,7 +376,7 @@ __device__ float chain_init(float* sm, const SmallParams& P, const float* q_row,
       if (wposT >= 0) sm[wposT] = v;
     }
   }
-  chain_sync<NW>(bar);
+  __syncwarp();
   int* meta = reinterpret_cast<int*>(sm + L.meta);
   int* wposv = reinterpret_cast<int*>(sm + L.wpos);
   int* wposTv = reinterpret_cast<int*>(sm + L.wposT);
@@ -424,15 +401,15 @@ __device__ float chain_init(float* sm, const SmallParams& P, const float* q_row,
     sm[wpos] = qv;
     if (wposT >= 0) sm[wposT] = qv;
   }
-  const float yv = stage_chunk<W, NW>(sm, P, ct, 0);
-  chain_sync<NW>(bar);
+  const float yv = stage_chunk<W>(sm, P, ct, 0);
+  __syncwarp();
   return yv;
 }
 
 // forward pass of the staged chunk; returns the network output of this thread's data point (point mode)
-template <int W, int NW>
-__device__ __forceinline__ float forward_chunk(float* sm, const SmallParams& P, int ct, int bar) {
-  using C = Cfg<W, NW>;
+template <int W>
+__device__ __forceinline__ float forward_chunk(float* sm, const SmallParams& P, int ct) {
+  using C = Cfg<W>;
   constexpr int PPL = C::PPL, NCS = C::NCS, WSW = C::WSW;
   const SmallLayout& L = P.lay;
   float* act = sm + L.act_base;
@@ -463,7 +440,7 @@ __device__ __forceinline__ float forward_chunk(float* sm, const SmallParams& P, 
     store8(act + L.h + j * NCS + c0, z);
     if (P.act == VIHMC_ACT_SINE) store8(act + L.da + j * NCS + c0, da);
   }
-  chain_sync<NW>(bar);
+  __syncwarp();
   for (int l = 1; l < P.n_hidden; ++l) {
     if (unit) {
       float z[PPL], da[PPL];
@@ -475,7 +452,7 @@ __device__ __forceinline__ float forward_chunk(float* sm, const SmallParams& P, 
       store8(act + L.h + (l * W + j) * NCS + c0, z);
       if (P.act == VIHMC_ACT_SINE) store8(act + L.da + (l * W + j) * NCS + c0, da);
     }
-    chain_sync<NW>(bar);
+    __syncwarp();
   }
   float o = 0.0f;
   if (ct < C::NC) {  // output layer, out_dim = 1
@@ -489,9 +466,9 @@ __device__ __forceinline__ float forward_chunk(float* sm, const SmallParams& P, 
 }
 
 // backward pass: writes the pre-activation gradients dz of every hidden layer (dO is already in smem)
-template <int W, int NW>
-__device__ __forceinline__ void backward_chunk(float* sm, const SmallParams& P, int ct, int bar) {
-  using C = Cfg<W, NW>;
+template <int W>
+__device__ __forceinline__ void backward_chunk(float* sm, const SmallParams& P, int ct) {
+  using C = Cfg<W>;
   constexpr int PPL = C::PPL, NCS = C::NCS, WSW = C::WSW;
   const SmallLayout& L = P.lay;
   float* act = sm + L.act_base;
@@ -507,7 +484,7 @@ __device__ __forceinline__ void backward_chunk(float* sm, const SmallParams& P, 
     for (int t = 0; t < PPL; ++t) dz[t] = wo * dO[t] * da[t];
     store8(act + L.dz + (top * W + j) * NCS + c0, dz);
   }
-  chain_sync<NW>(bar);
+  __syncwarp();
   for (int l = top; l >= 1; --l) {
     if (unit) {
       float acc[PPL], da[PPL];
@@ -519,17 +496,17 @@ __device__ __forceinline__ void backward_chunk(float* sm, const SmallParams& P, 
       for (int t = 0; t < PPL; ++t) acc[t] *= da[t];
       store8(act + L.dz + ((l - 1) * W + j) * NCS + c0, acc);
     }
-    chain_sync<NW>(bar);
+    __syncwarp();
   }
 }
 
 // phase B: thread = sampled coordinate; accumulates d loglik / d q_i of the staged chunk.  On the last
 // chunk the finished likelihood gradient of coordinate i goes straight to `consume(i, g_i)` (prior, kick,
 // drift, weight-table scatter: one pass, no round trip through sm[g]); earlier chunks park it in sm[g].
-template <int W, int NW, typename Consume>
+template <int W, typename Consume>
 __device__ __forceinline__ void phase_b(float* sm, const SmallParams& P, int ct, bool first_chunk, bool last_chunk,
                                         Consume&& consume) {
-  using C = Cfg<W, NW>;
+  using C = Cfg<W>;
   const SmallLayout& L = P.lay;
   const float* act = sm + L.act_base;
   const int* meta = reinterpret_cast<const int*>(sm + L.meta);
@@ -557,10 +534,10 @@ __device__ __forceinline__ void phase_b(float* sm, const SmallParams& P, int ct,
 
 // One gradient evaluation: consume(i, d loglik / d q_i) is called once per sampled coordinate (no prior
 // yet); returns this thread's share of the log-likelihood.  yv0 = the thread's target when N fits one chunk.
-template <int W, int NW, typename Consume>
-__device__ __forceinline__ float eval_likelihood_grad(float* sm, const SmallParams& P, const Likelihood lik, int ct, int bar,
-                                                      float yv0, Consume&& consume) {
-  using C = Cfg<W, NW>;
+template <int W, typename Consume>
+__device__ __forceinline__ float eval_likelihood_grad(float* sm, const SmallParams& P, const Likelihood lik, int ct, float yv0,
+                                                      Consume&& consume) {
+  using C = Cfg<W>;
   const SmallLayout& L = P.lay;
   float* act = sm + L.act_base;
   const int n_chunks = (int)((P.N + C::NC - 1) / C::NC);
@@ -568,20 +545,20 @@ __device__ __forceinline__ float eval_likelihood_grad(float* sm, const SmallPara
   for (int chunk = 0; chunk < n_chunks; ++chunk) {
     float yv = yv0;
     if (n_chunks > 1) {
-      yv = stage_chunk<W, NW>(sm, P, ct, chunk);
-      chain_sync<NW>(bar);
+      yv = stage_chunk<W>(sm, P, ct, chunk);
+      __syncwarp();
     }
-    const float o = forward_chunk<W, NW>(sm, P, ct, bar);
+    const float o = forward_chunk<W>(sm, P, ct);
     if (ct < C::NC) {
       const bool valid = (long long)chunk * C::NC + ct < P.N;
       const float r = o - yv;
       act[L.dO + ct] = valid ? -lik.prec * r : 0.0f;
       if (valid) ll_lane += lik.ll_const - lik.half_prec * r * r;
     }
-    chain_sync<NW>(bar);
-    backward_chunk<W, NW>(sm, P, ct, bar);
-    phase_b<W, NW>(sm, P, ct, chunk == 0, chunk == n_chunks - 1, consume);
-    chain_sync<NW>(bar);
+    __syncwarp();
+    backward_chunk<W>(sm, P, ct);
+    phase_b<W>(sm, P, ct, chunk == 0, chunk == n_chunks - 1, consume);
+    __syncwarp();
   }
   return ll_lane;
 }
@@ -767,7 +744,7 @@ __device__ __forceinline__ float eval_fast(float* sm, const SmallParams& P, cons
     }
   }
   __syncwarp();
-  phase_b<W, 1>(sm, P, ct, true, true, consume);
+  phase_b<W>(sm, P, ct, true, true, consume);
   __syncwarp();
   return ll_lane;
 }
@@ -1065,19 +1042,19 @@ __device__ __forceinline__ float eval_fast2(float* sm, const SmallParams& P, con
 // ------------------------------------------------------------------------------------------------
 // kernel 1: log-posterior value + gradient for C chains (vihmc_logp_grad, MLP small path)
 // ------------------------------------------------------------------------------------------------
-template <int W, int NW, int FAST>
+template <int W, int FAST>
 __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHMC_SMALL_MINBLOCKS) mlp_small_logp_grad_kernel(SmallParams P, long long C,
                                                                                          const float* __restrict__ q,
                                                                                          float* __restrict__ logp,
                                                                                          float* __restrict__ grad) {
   extern __shared__ __align__(16) float smem[];
-  constexpr int T = Cfg<W, NW>::T;
-  const int ct = threadIdx.x % T, slot = threadIdx.x / T, bar = 1 + slot;
+  constexpr int T = Cfg<W>::T;
+  const int ct = threadIdx.x % T, slot = threadIdx.x / T;
   const long long chain = (long long)blockIdx.x * (blockDim.x / T) + slot;
   if (chain >= C) return;
   const SmallLayout& L = P.lay;
   float* sm = smem + (size_t)slot * L.total;
-  const float yv0 = chain_init<W, NW>(sm, P, q + chain * P.d, ct, bar, chain);
+  const float yv0 = chain_init<W>(sm, P, q + chain * P.d, ct, chain);
   const Likelihood lik = make_likelihood(P.loss, P.tau_out);
   float lp_lane = 0.0f;
   auto consume = [&](int i, float gl) {
@@ -1096,63 +1073,63 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
     fast_setup<W>(sm, ct, yv0, F);
     ll_lane = eval_fast<W>(sm, P, lik, ct, F, consume);
   } else {
-    ll_lane = eval_likelihood_grad<W, NW>(sm, P, lik, ct, bar, yv0, consume);
+    ll_lane = eval_likelihood_grad<W>(sm, P, lik, ct, yv0, consume);
   }
-  const float total = chain_sum<NW>(fmaf(lp_lane, P.inv_prior_scale, ll_lane), sm + L.red, ct, bar) + P.prior_log_norm * P.inv_prior_scale;
+  const float total = warp_sum(fmaf(lp_lane, P.inv_prior_scale, ll_lane)) + P.prior_log_norm * P.inv_prior_scale;
   if (ct == 0) logp[chain] = total;
 }
 
 // ------------------------------------------------------------------------------------------------
 // kernel 1b: forward only (vihmc_predict, MLP small path): out[C, N]
 // ------------------------------------------------------------------------------------------------
-template <int W, int NW>
+template <int W>
 __global__ void __launch_bounds__(128) mlp_small_predict_kernel(SmallParams P, long long C, const float* __restrict__ q,
                                                                 float* __restrict__ out) {
   extern __shared__ __align__(16) float smem[];
-  using Cf = Cfg<W, NW>;
+  using Cf = Cfg<W>;
   constexpr int T = Cf::T;
-  const int ct = threadIdx.x % T, slot = threadIdx.x / T, bar = 1 + slot;
+  const int ct = threadIdx.x % T, slot = threadIdx.x / T;
   const long long chain = (long long)blockIdx.x * (blockDim.x / T) + slot;
   if (chain >= C) return;
   float* sm = smem + (size_t)slot * P.lay.total;
-  chain_init<W, NW>(sm, P, q + chain * P.d, ct, bar, chain);
+  chain_init<W>(sm, P, q + chain * P.d, ct, chain);
   const int n_chunks = (int)((P.N + Cf::NC - 1) / Cf::NC);
   for (int chunk = 0; chunk < n_chunks; ++chunk) {
     if (chunk > 0) {
-      stage_chunk<W, NW>(sm, P, ct, chunk);
-      chain_sync<NW>(bar);
+      stage_chunk<W>(sm, P, ct, chunk);
+      __syncwarp();
     }
-    const float o = forward_chunk<W, NW>(sm, P, ct, bar);
+    const float o = forward_chunk<W>(sm, P, ct);
     const long long n = (long long)chunk * Cf::NC + ct;
     if (ct < Cf::NC && n < P.N) out[chain * P.N + n] = o;
-    chain_sync<NW>(bar);
+    __syncwarp();
   }
 }
 
 // ------------------------------------------------------------------------------------------------
 // kernel 1c: sensitivity scores of the VI -> HMC split selector (vihmc_mlp_sensitivity)
 // Neural_network/VI/sensitivity.py:71-126: S_i = sigma_i^2 * mean_n (d o(x_n) / d w_i)^2 at w = the VI means.
-// One CTA (one warp per NW) per chunk of data points: forward, backward with d loss / d o = 1, then phase B with the
+// One CTA (one warp) per chunk of data points: forward, backward with d loss / d o = 1, then phase B with the
 // SQUARED per-point products; partial[chunk, i] = sum over the chunk's points, summed in fixed order by the finish kernel.
 // ------------------------------------------------------------------------------------------------
-template <int W, int NW>
+template <int W>
 __global__ void __launch_bounds__(128) mlp_small_sensitivity_kernel(SmallParams P, const float* __restrict__ w,
                                                                     float* __restrict__ partial) {
   extern __shared__ __align__(16) float sm[];
-  using Cf = Cfg<W, NW>;
-  const int ct = threadIdx.x, bar = 1;
+  using Cf = Cfg<W>;
+  const int ct = threadIdx.x;
   const int chunk = blockIdx.x;
   const SmallLayout& L = P.lay;
-  chain_init<W, NW>(sm, P, w, ct, bar);
+  chain_init<W>(sm, P, w, ct);
   if (chunk > 0) {
-    stage_chunk<W, NW>(sm, P, ct, chunk);
-    chain_sync<NW>(bar);
+    stage_chunk<W>(sm, P, ct, chunk);
+    __syncwarp();
   }
-  forward_chunk<W, NW>(sm, P, ct, bar);
+  forward_chunk<W>(sm, P, ct);
   float* act = sm + L.act_base;
   if (ct < Cf::NC) act[L.dO + ct] = ((long long)chunk * Cf::NC + ct < P.N) ? 1.0f : 0.0f;   // d o / d o
-  chain_sync<NW>(bar);
-  backward_chunk<W, NW>(sm, P, ct, bar);
+  __syncwarp();
+  backward_chunk<W>(sm, P, ct);
   const int* meta = reinterpret_cast<const int*>(sm + L.meta);
   for (int i = ct; i < (int)P.d; i += Cf::T) {
     const int m = meta[i];
@@ -1191,20 +1168,19 @@ struct SampleArgs {
 
 // MASS: diagonal mass m = A.inv_mass (hamiltorch's 1-D inv_mass).  p = fl(z s_i), ke = 0.5 sum p fl(m_i p), drift
 // q += fl(fl(eps m_i) p); with MASS = false the code is exactly the identity-mass kernel.
-template <int W, int NW, int FAST, bool MASS>
+template <int W, int FAST, bool MASS>
 __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHMC_SMALL_MINBLOCKS) mlp_small_sample_kernel(SmallParams P, SampleArgs A) {
   extern __shared__ __align__(16) float smem[];
-  constexpr int T = Cfg<W, NW>::T;
-  const int ct = threadIdx.x % T, slot = threadIdx.x / T, bar = 1 + slot;
+  constexpr int T = Cfg<W>::T;
+  const int ct = threadIdx.x % T, slot = threadIdx.x / T;
   const long long chain = (long long)blockIdx.x * (blockDim.x / T) + slot;
   if (chain >= A.C) return;
   const SmallLayout& L = P.lay;
   float* sm = smem + (size_t)slot * L.total;
-  float* red = sm + L.red;
   const int d = (int)P.d;
   const long long C = A.C;
   const float* q0 = A.q0 + chain * d;
-  const float yv0 = chain_init<W, NW, MASS>(sm, P, q0, ct, bar, chain, A.inv_mass);
+  const float yv0 = chain_init<W, MASS>(sm, P, q0, ct, chain, A.inv_mass);
   FastRegs F;
   if constexpr (FAST != 0) fast_setup<W>(sm, ct, yv0, F);
   if constexpr (FAST >= 2) fast2_setup<W>(sm, P, ct);
@@ -1281,14 +1257,14 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
           }
         }
       }
-      chain_sync<NW>(bar);
+      __syncwarp();
       for (int i = ct; i < d; i += T) {
         const float qv = sm[L.q + i];
         sm[wposv[i]] = qv;
         const int wt = wposTv[i];
         if (wt >= 0) sm[wt] = qv;
       }
-      chain_sync<NW>(bar);
+      __syncwarp();
     }
     // ---- momentum ----
     float ke = 0.0f;
@@ -1319,8 +1295,8 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
           }
       }
     }
-    const float ke0 = 0.5f * chain_sum<NW>(ke, red, ct, bar);
-    chain_sync<NW>(bar);
+    const float ke0 = 0.5f * warp_sum(ke);
+    __syncwarp();
 
     // ---- trajectory: evaluation s = 0 yields H0 and the first half kick; s = nsteps yields H1 ----
     const float half_eps = 0.5f * eps;
@@ -1362,9 +1338,9 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
         }
         __syncwarp();
         if (first || last) {
-          const float lp = chain_sum<NW>(fmaf(lp_lane, P.inv_prior_scale, ll3), red, ct, bar) + log_norm;
+          const float lp = warp_sum(fmaf(lp_lane, P.inv_prior_scale, ll3)) + log_norm;
           if (first) logp0 = lp;
-          if (last) { logp1 = lp; ke1 = 0.5f * chain_sum<NW>(ke_lane, red, ct, bar); }
+          if (last) { logp1 = lp; ke1 = 0.5f * warp_sum(ke_lane); }
         }
         continue;
       }
@@ -1391,13 +1367,13 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
       float ll_lane;
       if constexpr (FAST == 2) ll_lane = eval_fast2<W>(sm, P, lik, ct, F, consume);
       else if constexpr (FAST == 1) ll_lane = eval_fast<W>(sm, P, lik, ct, F, consume);
-      else ll_lane = eval_likelihood_grad<W, NW>(sm, P, lik, ct, bar, yv0, consume);
+      else ll_lane = eval_likelihood_grad<W>(sm, P, lik, ct, yv0, consume);
       if (first || last) {
-        const float lp = chain_sum<NW>(fmaf(lp_lane, P.inv_prior_scale, ll_lane), red, ct, bar) + log_norm;
+        const float lp = warp_sum(fmaf(lp_lane, P.inv_prior_scale, ll_lane)) + log_norm;
         if (first) logp0 = lp;
-        if (last) { logp1 = lp; ke1 = 0.5f * chain_sum<NW>(ke_lane, red, ct, bar); }
+        if (last) { logp1 = lp; ke1 = 0.5f * warp_sum(ke_lane); }
       }
-      chain_sync<NW>(bar);
+      __syncwarp();
     }
     if constexpr (FAST == 3) {
 #pragma unroll
@@ -1457,7 +1433,7 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
       }
       if (n == burn) eps = eps_bar;
     }
-    chain_sync<NW>(bar);
+    __syncwarp();
   }
   if (A.step_sizes != nullptr && ct == 0) A.step_sizes[chain] = eps;
 }
@@ -1468,7 +1444,7 @@ __global__ void __launch_bounds__(128, FAST >= 2 ? VIHMC_SMALL_MINBLOCKS2 : VIHM
 enum SmallOp { kOpLogpGrad = 0, kOpPredict = 1, kOpSample = 2, kOpSensitivity = 3 };
 
 struct SmallLaunch {
-  int warps_per_chain, chains_per_block, blocks;
+  int chains_per_block, blocks;
   int fast;   // specialised 1-W-W-1 tanh single-chunk evaluation: 1 = eval_fast, 2 = eval_fast2 (register partial sums, W <= 16)
   size_t smem;
   long long C;
@@ -1485,26 +1461,26 @@ static int set_smem(K kernel, size_t bytes) {
   return VIHMC_OK;
 }
 
-template <int W, int NW, int FAST, bool MASS = false>
+template <int W, int FAST, bool MASS = false>
 static int launch_small_wn(SmallOp op, const SmallParams& P, const SmallLaunch& a, cudaStream_t st) {
-  const int threads = a.chains_per_block * 32 * NW;
+  const int threads = a.chains_per_block * 32;
   if (op == kOpLogpGrad) {
-    auto k = mlp_small_logp_grad_kernel<W, NW, FAST>;
+    auto k = mlp_small_logp_grad_kernel<W, FAST>;
     if (int rc = set_smem(k, a.smem)) return rc;
     k<<<a.blocks, threads, a.smem, st>>>(P, a.C, a.q, a.logp, a.grad);
     VIHMC_LAUNCH_OK("mlp_small_logp_grad_kernel");
   } else if (op == kOpSensitivity) {   // q = weights, out = partial sums [blocks, d]
-    auto k = mlp_small_sensitivity_kernel<W, NW>;
+    auto k = mlp_small_sensitivity_kernel<W>;
     if (int rc = set_smem(k, a.smem)) return rc;
-    k<<<a.blocks, 32 * NW, a.smem, st>>>(P, a.q, a.out);
+    k<<<a.blocks, 32, a.smem, st>>>(P, a.q, a.out);
     VIHMC_LAUNCH_OK("mlp_small_sensitivity_kernel");
   } else if (op == kOpPredict) {
-    auto k = mlp_small_predict_kernel<W, NW>;
+    auto k = mlp_small_predict_kernel<W>;
     if (int rc = set_smem(k, a.smem)) return rc;
     k<<<a.blocks, threads, a.smem, st>>>(P, a.C, a.q, a.out);
     VIHMC_LAUNCH_OK("mlp_small_predict_kernel");
   } else {
-    auto k = mlp_small_sample_kernel<W, NW, FAST, MASS>;
+    auto k = mlp_small_sample_kernel<W, FAST, MASS>;
     if (int rc = set_smem(k, a.smem)) return rc;
     k<<<a.blocks, threads, a.smem, st>>>(P, a.A);
     VIHMC_LAUNCH_OK("mlp_small_sample_kernel");
@@ -1513,21 +1489,20 @@ static int launch_small_wn(SmallOp op, const SmallParams& P, const SmallLaunch& 
 }
 
 // the sampler with a diagonal mass takes the MASS instantiation of the same variant (only the sample kernel has one)
-template <int W, int NW, int FAST>
+template <int W, int FAST>
 static int launch_small_wm(SmallOp op, const SmallParams& P, const SmallLaunch& a, cudaStream_t st) {
-  if (op == kOpSample && a.A.inv_mass != nullptr) return launch_small_wn<W, NW, FAST, true>(op, P, a, st);
-  return launch_small_wn<W, NW, FAST, false>(op, P, a, st);
+  if (op == kOpSample && a.A.inv_mass != nullptr) return launch_small_wn<W, FAST, true>(op, P, a, st);
+  return launch_small_wn<W, FAST, false>(op, P, a, st);
 }
 
 template <int W>
 static int launch_small_w(SmallOp op, const SmallParams& P, const SmallLaunch& a, cudaStream_t st) {
-  if (a.warps_per_chain == 2) return launch_small_wm<W, 2, 0>(op, P, a, st);
   if constexpr (W <= 16) {   // version 2 keeps 2 W quads in registers: widths above 16 stay on version 1
-    if (a.fast == 2 && op == kOpSample && P.d <= 32 * kRegRounds) return launch_small_wm<W, 1, 3>(op, P, a, st);
-    if (a.fast == 2) return launch_small_wm<W, 1, 2>(op, P, a, st);
+    if (a.fast == 2 && op == kOpSample && P.d <= 32 * kRegRounds) return launch_small_wm<W, 3>(op, P, a, st);
+    if (a.fast == 2) return launch_small_wm<W, 2>(op, P, a, st);
   }
-  if (a.fast) return launch_small_wm<W, 1, 1>(op, P, a, st);
-  return launch_small_wm<W, 1, 0>(op, P, a, st);
+  if (a.fast) return launch_small_wm<W, 1>(op, P, a, st);
+  return launch_small_wm<W, 0>(op, P, a, st);
 }
 
 }  // namespace vihmc
