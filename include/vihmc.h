@@ -311,8 +311,9 @@ VIHMC_API int vihmc_vi_epoch_end(const vihmc_vi_cfg* cfg, int64_t D, const float
  *   C[b][m, n] = sum_k opA[b][m, k] * opB[b][k, n],   b < batch
  * with opA[b][m,k] at A + b*a_bs + m*a_sm + k*a_sk, opB[b][k,n] at B + b*b_bs + k*b_sk + n*b_sn and C[b][m,n] at
  * C + b*c_bs + m*ldc + n (element strides, a batch stride of 0 shares the operand).  use_tensor_cores = 1 runs the
- * tcgen05 3xTF32 kernel (needs M >= 32, K >= 16), 0 the FP32 SIMT kernel.  K > 2048 with a non-NULL
- * splitk_scratch (ceil(K/1024) * batch * M * N floats) is split into 1024-deep slices summed in fixed order.
+ * tcgen05 3xTF32 kernel (needs M >= 32, K >= 16), 0 the FP32 SIMT kernel.  With the tensor cores, a non-NULL
+ * splitk_scratch (ceil(K/256) * batch * M * N floats) makes every K > 384 split into slices of about 256, whose partial
+ * products are summed in fixed order.
  */
 VIHMC_API int vihmc_gemm_batched(const float* A, int64_t a_bs, int64_t a_sm, int64_t a_sk, const float* B, int64_t b_bs,
                        int64_t b_sk, int64_t b_sn, float* C, int64_t c_bs, int64_t ldc, int32_t M, int32_t N, int32_t K,

@@ -1,5 +1,5 @@
 """Diagnostic (not collected by pytest): per-tensor error of the engine's BASELINE-size DeepONet gradient against the reference
-golden vectors and the fp64 twin, for the path selected by the environment (VIHMC_DENSE_SIMT / VIHMC_DENSE_NOFUSE / VIHMC_TC_TMEMA).
+golden vectors and the fp64 twin, for the path selected by the environment (VIHMC_DENSE_SIMT / VIHMC_DENSE_NOFUSE).
     python tests/diag_fullsize.py [full|vi]"""
 import os
 import sys

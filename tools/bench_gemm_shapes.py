@@ -19,7 +19,7 @@ def main():
     dZ = torch.randn(C, P, K, device=dev); H = torch.randn(C, P, K, device=dev)
     Pp = 10204
     G = torch.randn(C, N, Pp, device=dev)[:, :, :P]; xb = torch.randn(C, N, K, device=dev); xtr = torch.randn(C, P, K, device=dev)
-    out = {"lib": os.environ.get("VIHMC_LIB_PATH", "default"), "tmema": os.environ.get("VIHMC_TC_TMEMA", "1")}
+    out = {"lib": os.environ.get("VIHMC_LIB_PATH", "default")}
     out["dW_us"] = timed(lambda: engine.gemm_batched(dZ.transpose(1, 2), H))
     out["dxtr_us"] = timed(lambda: engine.gemm_batched(G.transpose(1, 2), xb))
     out["dxb_us"] = timed(lambda: engine.gemm_batched(G, xtr))

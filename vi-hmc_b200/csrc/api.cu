@@ -35,9 +35,9 @@ int vi_epoch_end(const vihmc_vi_cfg*, long long D, const float* valid_logp, int 
                  const float* rho, float* history, void* ws, size_t ws_bytes, cudaStream_t);
 bool dense_supported(const vihmc_problem* p);
 size_t dense_workspace_bytes(const vihmc_problem*, long long C);
-int dense_logp_grad(const vihmc_problem*, long long C, const float* q, float* logp, float* grad, void* ws, size_t ws_bytes,
-                    cudaStream_t);
-int dense_predict(const vihmc_problem*, long long C, const float* q, float* out, void* ws, size_t ws_bytes, cudaStream_t);
+// log-posterior (out == NULL) or predict (out != NULL) on the dense path
+int dense_run(const vihmc_problem*, long long C, const float* q, float* logp, float* grad, float* out, void* ws, size_t ws_bytes,
+              cudaStream_t);
 int dense_umma_probe(const float* a_img, const float* b_img, unsigned a_lbo, unsigned a_sbo, unsigned b_lbo, unsigned b_sbo,
                      unsigned a_type, unsigned b_type, unsigned idesc_extra, float* out, cudaStream_t);
 int dense_debug_tanh(int kind, const float* x, float* y, long long n, cudaStream_t st);
@@ -186,7 +186,7 @@ static size_t sampler_state_bytes(long long C, long long d, long long D_redraw =
 static int model_logp_grad(const vihmc_problem* p, long long C, const float* q, float* logp, float* grad, void* ws, size_t ws_bytes,
                            cudaStream_t st) {
   if (mlp_small_supported(p)) return mlp_small_logp_grad(p, C, q, logp, grad, st);
-  if (dense_supported(p)) return dense_logp_grad(p, C, q, logp, grad, ws, ws_bytes, st);
+  if (dense_supported(p)) return dense_run(p, C, q, logp, grad, nullptr, ws, ws_bytes, st);
   return fail(VIHMC_ERR_UNSUPPORTED, "no kernel for this architecture");
 }
 
@@ -261,7 +261,7 @@ int vihmc_predict(const vihmc_problem* prob, int64_t C, const float* q, float* o
   if (int rc = device_check()) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (mlp_small_supported(prob)) return mlp_small_predict(prob, C, q, out, st);
-  if (dense_supported(prob)) return dense_predict(prob, C, q, out, workspace, workspace_bytes, st);
+  if (dense_supported(prob)) return dense_run(prob, C, q, nullptr, nullptr, out, workspace, workspace_bytes, st);
   return fail(VIHMC_ERR_UNSUPPORTED, "no kernel for this architecture");
 }
 

@@ -232,12 +232,13 @@ static bool tensor_cores_enabled() {
 }
 
 template <int EPI>
-static int launch_gemm(const GemmArgs& g, int batch, cudaStream_t st, float* scratch = nullptr, int force = -1,
-                       float* rowsum_part = nullptr, float* rowsum_out = nullptr, long long rowsum_bs = 0, int* rowsum_done = nullptr) {
+static int launch_gemm(const GemmArgs& g, int batch, cudaStream_t st, float* scratch = nullptr, long long scratch_floats = 0,
+                       int force = -1, float* rowsum_part = nullptr, float* rowsum_out = nullptr, long long rowsum_bs = 0,
+                       int* rowsum_done = nullptr) {
   if (g.M < 1 || g.N < 1 || g.K < 1 || batch < 1) return fail(VIHMC_ERR_INVALID, "gemm: empty problem");
   if (batch > 65535) return fail(VIHMC_ERR_UNSUPPORTED, "gemm: batch > 65535");
   const bool tc = force < 0 ? tensor_cores_enabled() && tc_gemm_eligible(g) : force == 1;
-  if (tc) return launch_tc_gemm<EPI>(g, batch, st, scratch, rowsum_part, rowsum_out, rowsum_bs, rowsum_done);
+  if (tc) return launch_tc_gemm<EPI>(g, batch, st, scratch, scratch_floats, rowsum_part, rowsum_out, rowsum_bs, rowsum_done);
   if (EPI == EPI_STORE && force < 0 && tensor_cores_enabled() && g.M == 1) {
     // A single output row over a long reduction (the output layer's weight gradient dW[1, in] = dz^T[1, R] a[R, in] of the
     // wide-BNN config: 22 ms per evaluation on the SIMT kernel, a third of the whole gradient): run the transposed problem
@@ -246,7 +247,7 @@ static int launch_gemm(const GemmArgs& g, int batch, cudaStream_t st, float* scr
     t.A = g.B; t.a_bs = g.b_bs; t.a_sm = g.b_sn; t.a_sk = g.b_sk;
     t.B = g.A; t.b_bs = g.a_bs; t.b_sk = g.a_sk; t.b_sn = g.a_sm;
     t.M = g.N; t.N = 1; t.ldc = 1;
-    if (tc_gemm_eligible(t)) return launch_tc_gemm<EPI>(t, batch, st, scratch);   // no fused row sums: opA is not dz any more
+    if (tc_gemm_eligible(t)) return launch_tc_gemm<EPI>(t, batch, st, scratch, scratch_floats);   // no fused row sums: opA is not dz any more
   }
   if (EPI != EPI_HEAD && force < 0 && g.K <= SMALLK_MAX && g.N >= 16) {
     const long long threads = (long long)g.M * ((g.N + 3) / 4);
@@ -538,12 +539,30 @@ static int stack_forward_fused(const Stack& s, const float* input, long long R, 
   return VIHMC_OK;
 }
 
+// weight gradient of layer l, dW[o,i] = sum_r dz[r,o] * a_in[r,i], and its bias gradient = column sums of dz = row sums of
+// opA: the tensor-core GEMM reads them off its operand stream when it can (MN-major A), launch_colsum sums them otherwise;
+// `part` holds the bias partials either way
+static int layer_weight_grad(const Stack& s, int l, const float* input, long long R, float* const* acts, const float* dz, float* dWf,
+                             long long Dp, float* part, int Cb, float* scratch, long long scratch_floats, cudaStream_t st) {
+  const int in = s.in_of(l), out = s.dims[l];
+  GemmArgs g{};
+  g.A = dz; g.a_bs = R * out; g.a_sm = 1; g.a_sk = out;            // opA[m=o,k=r] = dz[r,o]
+  g.B = l == 0 ? input : acts[l - 1]; g.b_bs = l == 0 ? 0 : R * in; g.b_sk = in; g.b_sn = 1;
+  g.C = dWf + s.w_off[l]; g.c_bs = Dp; g.ldc = s.ldw[l];
+  g.M = out; g.N = in; g.K = (int)R;
+  float* bias = s.has_bias[l] ? dWf + s.b_off[l] : nullptr;
+  int bias_done = 0;
+  if (int rc = launch_gemm<EPI_STORE>(g, Cb, st, scratch, scratch_floats, -1, bias ? part : nullptr, bias, Dp, &bias_done)) return rc;
+  if (bias != nullptr && !bias_done)
+    if (int rc = launch_colsum(dz, R * out, R, out, out, part, bias, Dp, Cb, st)) return rc;
+  return VIHMC_OK;
+}
+
 // backward of one stack with the data pass in ONE kernel (fused_stack.cuh): dzs[top] holds d/d(pre-activation of the last
 // layer) on entry, dzs[l < top] are written by the kernel; the weight / bias gradients follow as one GEMM per layer.
 static int stack_backward_fused(const Stack& s, const float* input, long long R, const float* Wf, float* dWf, long long Dp,
                                 float* const* acts, float* const* dzs, int act, int Cb, float* img, float* bias_part, float* scratch,
-                                cudaStream_t st) {
-  const int top = s.n_layers - 1;
+                                long long scratch_floats, cudaStream_t st) {
   fused::ImgTable t{};
   t.n = s.n_layers - 1;
   for (int l = 1; l < s.n_layers; ++l) t.L[l - 1] = fused::ImgLayer{s.w_off[l], s.in_of(l), s.dims[l], 1, s.ldw[l]};   // W_l^T
@@ -561,30 +580,11 @@ static int stack_backward_fused(const Stack& s, const float* input, long long R,
   if (act == VIHMC_ACT_TANH) { if (int rc = launch(fused::fused_backward_kernel<VIHMC_ACT_TANH>)) return rc; }
   else { if (int rc = launch(fused::fused_backward_kernel<VIHMC_ACT_RELU>)) return rc; }
   VIHMC_LAUNCH_OK("fused_backward_kernel");
-  for (int l = top; l >= 0; --l) {
-    const int in = s.in_of(l), out = s.dims[l];
-    GemmArgs g{};   // dW[o,i] = sum_r dz[r,o] * a_in[r,i]
-    g.A = dzs[l]; g.a_bs = R * out; g.a_sm = 1; g.a_sk = out;
-    g.B = l == 0 ? input : acts[l - 1]; g.b_bs = l == 0 ? 0 : R * in; g.b_sk = in; g.b_sn = 1;
-    g.C = dWf + s.w_off[l]; g.c_bs = Dp; g.ldc = s.ldw[l];
-    g.M = out; g.N = in; g.K = (int)R;
-    int bias_done = 0;
-    if (int rc = launch_gemm<EPI_STORE>(g, Cb, st, scratch, -1, bias_part, dWf + s.b_off[l], Dp, &bias_done)) return rc;
-    if (!bias_done)
-      if (int rc = launch_colsum(dzs[l], R * out, R, out, out, bias_part, dWf + s.b_off[l], Dp, Cb, st)) return rc;
-  }
+  for (int l = s.n_layers - 1; l >= 0; --l)
+    if (int rc = layer_weight_grad(s, l, input, R, acts, dzs[l], dWf, Dp, bias_part, Cb, scratch, scratch_floats, st)) return rc;
   return VIHMC_OK;
 }
 
-// VIHMC_DENSE_FWD3=0 keeps the forward pass on the 3xTF32 kernels (A/B runs; that path carries the tensor core's
-// accumulate-truncation bias, see xgemm.cuh)
-static bool fwd3_enabled() {
-  static const bool on = []() {
-    const char* e = getenv("VIHMC_DENSE_FWD3");
-    return !(e != nullptr && e[0] == '0');
-  }();
-  return on;   // independent of VIHMC_DENSE_SIMT, so that "exact forward + FP32-SIMT backward" can be measured (error attribution)
-}
 static bool fwd3_eligible(const Stack& s) {
   if (s.n_layers < 2 || s.in_dim > xg::XK) return false;
   for (int l = 0; l < s.n_layers; ++l)
@@ -656,6 +656,10 @@ static int launch_head3(const DensePlan& pl, int Cb, const unsigned char* a_img,
   return VIHMC_OK;
 }
 
+// dBout = G Tout writes 400 KB per slice and chain: 512-deep slices halve that traffic (their share of the BASELINE-size
+// gradient error stays below 2e-6, tests/diag_fullsize.py)
+constexpr int kDBoutChunk = 512;
+
 static int make_plan(const vihmc_problem* p, DensePlan& pl) {
   pl.deeponet = p->model_kind == VIHMC_MODEL_DEEPONET;
   pl.N = p->N;
@@ -694,19 +698,16 @@ static int make_plan(const vihmc_problem* p, DensePlan& pl) {
   pl.loss_tiles = (pl.N + 255) / 256;
   const long long tiles = pl.deeponet ? pl.head_tiles : pl.loss_tiles;
   const long long G = pl.deeponet ? pl.N * pl.Pp : pl.N;
-  pl.scratch_per_chain = 0;   // split-K partials of the largest weight-gradient GEMM
-  for (int l = 0; l < pl.a.n_layers; ++l) {
-    const long long f = splitk_scratch_floats(pl.a.dims[l], pl.a.in_of(l), (int)pl.N, 1);
-    pl.scratch_per_chain = f > pl.scratch_per_chain ? f : pl.scratch_per_chain;
-  }
-  for (int l = 0; l < pl.b.n_layers; ++l) {
-    const long long f = splitk_scratch_floats(pl.b.dims[l], pl.b.in_of(l), (int)pl.P, 1);
-    pl.scratch_per_chain = f > pl.scratch_per_chain ? f : pl.scratch_per_chain;
-  }
+  pl.scratch_per_chain = 0;   // split-K partials of the largest product that can be split, at the most slices it can take
+  auto budget = [&](int M, int N, long long K, int kc_hint) {
+    const long long slices = splitk_max_slices((int)K, kc_hint);
+    if (slices > 1 && slices * M * N > pl.scratch_per_chain) pl.scratch_per_chain = slices * M * N;
+  };
+  for (int l = 0; l < pl.a.n_layers; ++l) budget(pl.a.dims[l], pl.a.in_of(l), pl.N, 0);   // weight gradients
+  for (int l = 0; l < pl.b.n_layers; ++l) budget(pl.b.dims[l], pl.b.in_of(l), pl.P, 0);
   if (pl.deeponet) {   // dBout = G Tout reduces over the P trunk points, dTout = G^T Bout over the N functions
-    const long long f = splitk_scratch_floats((int)pl.N, pl.K, (int)pl.P, 1), f2 = splitk_scratch_floats((int)pl.P, pl.K, (int)pl.N, 1);
-    pl.scratch_per_chain = f > pl.scratch_per_chain ? f : pl.scratch_per_chain;
-    pl.scratch_per_chain = f2 > pl.scratch_per_chain ? f2 : pl.scratch_per_chain;
+    budget((int)pl.N, pl.K, pl.P, kDBoutChunk);
+    budget((int)pl.P, pl.K, pl.N, 0);
   }
   // fused kernels (DeepONet stacks): weight images (the two stacks use the buffer one after the other), dz of every layer
   pl.fuse_a = pl.deeponet && fused_eligible(pl.a);
@@ -722,7 +723,7 @@ static int make_plan(const vihmc_problem* p, DensePlan& pl) {
     const long long wa = pl.a.max_width();
     pl.dzall_floats += (long long)(pl.a.n_layers - 1) * (pl.N * wa + 64) + ((pl.N + 127) / 128 + 16) * wa + 64;
   }
-  pl.fwd3 = pl.deeponet && fwd3_enabled() && fwd3_eligible(pl.a) && fwd3_eligible(pl.b) && pl.K <= xg::XK;
+  pl.fwd3 = pl.deeponet && fwd3_eligible(pl.a) && fwd3_eligible(pl.b) && pl.K <= xg::XK;
   pl.m_tiles = (int)((pl.N + 127) / 128);
   pl.p_tiles128 = (int)((pl.P + 127) / 128);
   pl.wimg3_floats = pl.ximg_a_floats = pl.ximg_b_floats = pl.xsc_floats = 0;
@@ -779,9 +780,10 @@ struct Bump {
 };
 }  // namespace
 
-// forward of one stack for Cb chains: in [R, in_dim] shared -> acts[l] [Cb, R, dims[l]]   (D = padded per-chain stride of Wf)
+// forward of one stack for Cb chains: in [R, in_dim] shared -> acts[l] [Cb, R, dims[l]]   (D = padded per-chain stride of Wf);
+// no activation on the last layer
 static int stack_forward(const Stack& s, const float* input, long long R, const float* Wf, long long D, float* const* acts,
-                         int act, bool act_on_last, int Cb, cudaStream_t st) {
+                         int act, int Cb, cudaStream_t st) {
   for (int l = 0; l < s.n_layers; ++l) {
     GemmArgs g{};
     const int in = s.in_of(l), out = s.dims[l];
@@ -790,10 +792,9 @@ static int stack_forward(const Stack& s, const float* input, long long R, const 
     g.B = Wf + s.w_off[l]; g.b_bs = D; g.b_sk = 1; g.b_sn = s.ldw[l];   // opB[k,n] = W[n,k]
     g.C = acts[l]; g.c_bs = R * out; g.ldc = out;
     g.M = (int)R; g.N = out; g.K = in;
-    const bool last = l == s.n_layers - 1;
     if (s.has_bias[l]) {
       g.bias = Wf + s.b_off[l]; g.bias_bs = D;
-      g.act = (last && !act_on_last) ? -1 : act;
+      g.act = l == s.n_layers - 1 ? -1 : act;
       if (int rc = launch_gemm<EPI_BIAS_ACT>(g, Cb, st)) return rc;
     } else {
       if (int rc = launch_gemm<EPI_STORE>(g, Cb, st)) return rc;
@@ -804,22 +805,12 @@ static int stack_forward(const Stack& s, const float* input, long long R, const 
 
 // backward of one stack: dz holds d/d(pre-activation of the last layer) [Cb, R, dims[last]] on entry.
 static int stack_backward(const Stack& s, const float* input, long long R, const float* Wf, float* dWf, long long D,
-                          float* const* acts, float* dz_cur, float* dz_other, int act, int Cb, cudaStream_t st, float* scratch) {
+                          float* const* acts, float* dz_cur, float* dz_other, int act, int Cb, float* scratch, long long scratch_floats,
+                          cudaStream_t st) {
   for (int l = s.n_layers - 1; l >= 0; --l) {
     const int in = s.in_of(l), out = s.dims[l];
-    // dW[o,i] = sum_r dz[r,o] * a_in[r,i]
-    GemmArgs g{};
-    g.A = dz_cur; g.a_bs = R * out; g.a_sm = 1; g.a_sk = out;            // opA[m=o,k=r] = dz[r,o]
-    g.B = l == 0 ? input : acts[l - 1]; g.b_bs = l == 0 ? 0 : R * in; g.b_sk = in; g.b_sn = 1;
-    g.C = dWf + s.w_off[l]; g.c_bs = D; g.ldc = s.ldw[l];
-    g.M = out; g.N = in; g.K = (int)R;
-    // bias gradient = column sums of dz = row sums of opA: the tensor-core GEMM reads them off its operand stream when
-    // it can (MN-major A); dz_other is free until the dX GEMM below writes it and holds the partials either way
-    int bias_done = 0;
-    if (int rc = launch_gemm<EPI_STORE>(g, Cb, st, scratch, -1, s.has_bias[l] ? dz_other : nullptr,
-                                        s.has_bias[l] ? dWf + s.b_off[l] : nullptr, D, &bias_done)) return rc;
-    if (s.has_bias[l] && !bias_done)
-      if (int rc = launch_colsum(dz_cur, R * out, R, out, out, dz_other, dWf + s.b_off[l], D, Cb, st)) return rc;
+    // dz_other is free until the dX GEMM below writes it: it holds the bias partials
+    if (int rc = layer_weight_grad(s, l, input, R, acts, dz_cur, dWf, D, dz_other, Cb, scratch, scratch_floats, st)) return rc;
     if (l > 0) {
       // dz_prev[r,i] = (sum_o dz[r,o] W[o,i]) * act'(a_{l-1}[r,i])
       GemmArgs h{};
@@ -835,22 +826,35 @@ static int stack_backward(const Stack& s, const float* input, long long R, const
   return VIHMC_OK;
 }
 
-// chain-independent buffers at the head of the workspace: pad map, trunk features, padded targets
+// forward of one stack of the plan: through fused_forward3_kernel when the plan runs both DeepONet stacks there (with the
+// operand image and row scales of the last layer's output for head3_kernel), else through the fused 3xTF32 kernel when this
+// stack is eligible (`fused`), else one GEMM per layer
+static int stack_forward_any(const DensePlan& pl, const Stack& s, bool fused, const float* input, long long R, const float* Wf,
+                             float* const* acts, int act, int Cb, float* img, unsigned char* wimg3, unsigned char* out_img,
+                             float* out_scales, cudaStream_t st) {
+  if (pl.fwd3) return stack_forward3(s, input, R, Wf, pl.Dp, acts, act, Cb, wimg3, out_img, out_scales, st);
+  if (fused) return stack_forward_fused(s, input, R, Wf, pl.Dp, acts, act, Cb, img, st);
+  return stack_forward(s, input, R, Wf, pl.Dp, acts, act, Cb, st);
+}
+
+// chain-independent buffers at the head of the workspace: pad map, trunk features, the targets the DeepONet head reads
 struct SharedBufs {
   const int* pad_map;
   const float* trunk_in;
-  const float* y_pad;   // [N, Pp] (DeepONet) or p->y
+  const float* y_pad;   // log-posterior: [N, Pp] (DeepONet) or p->y; predict: a zero row (HEAD epilogue) or null (head3_kernel)
+  long long ld_y;       // row stride of y_pad: Pp, or 0 for the zero row
   float* batch_base;
 };
 
-static int prepare_shared(const vihmc_problem* p, const DensePlan& pl, void* ws, bool need_targets, cudaStream_t st, SharedBufs& sb) {
+static int prepare_shared(const vihmc_problem* p, const DensePlan& pl, void* ws, bool predict, cudaStream_t st, SharedBufs& sb) {
   Bump bump(static_cast<float*>(ws));
   int* map = reinterpret_cast<int*>(bump.take(pl.D));
   pad_map_kernel<<<(unsigned)((pl.D + 255) / 256), 256, 0, st>>>(pl.tbl, pl.D, map);
   VIHMC_LAUNCH_OK("pad_map_kernel");
   sb.pad_map = map;
   sb.trunk_in = nullptr;
-  sb.y_pad = p->y;
+  sb.y_pad = predict ? nullptr : p->y;
+  sb.ld_y = pl.Pp;
   if (pl.deeponet) {
     if (p->impose_bc) {
       float* feats = bump.take(pl.P * 5);
@@ -860,14 +864,17 @@ static int prepare_shared(const vihmc_problem* p, const DensePlan& pl, void* ws,
     } else {
       sb.trunk_in = p->x2;
     }
-    if (need_targets) {
-      if (pl.Pp != pl.P) {   // rows of the targets on 16-byte boundaries: the head epilogue reads them with float4 loads
-        float* yp = bump.take(pl.N * pl.Pp);
-        VIHMC_CUDA_OK(cudaMemsetAsync(yp, 0, sizeof(float) * pl.N * pl.Pp, st));
-        VIHMC_CUDA_OK(cudaMemcpy2DAsync(yp, sizeof(float) * pl.Pp, p->y, sizeof(float) * pl.P, sizeof(float) * pl.P, (size_t)pl.N,
-                                        cudaMemcpyDeviceToDevice, st));
-        sb.y_pad = yp;
-      }
+    if (!predict && pl.Pp != pl.P) {   // rows of the targets on 16-byte boundaries: the head epilogue reads them with float4 loads
+      float* yp = bump.take(pl.N * pl.Pp);
+      VIHMC_CUDA_OK(cudaMemsetAsync(yp, 0, sizeof(float) * pl.N * pl.Pp, st));
+      VIHMC_CUDA_OK(cudaMemcpy2DAsync(yp, sizeof(float) * pl.Pp, p->y, sizeof(float) * pl.P, sizeof(float) * pl.P, (size_t)pl.N,
+                                      cudaMemcpyDeviceToDevice, st));
+      sb.y_pad = yp;
+    } else if (predict && !pl.fwd3) {   // the HEAD epilogue with prec = -1 against zero targets computes the outputs themselves
+      float* zero_row = bump.take(pl.Pp);
+      VIHMC_CUDA_OK(cudaMemsetAsync(zero_row, 0, sizeof(float) * pl.Pp, st));
+      sb.y_pad = zero_row;
+      sb.ld_y = 0;
     }
   }
   sb.batch_base = bump.take(0);
@@ -893,28 +900,32 @@ static int scatter_padded(const vihmc_problem* p, const DensePlan& pl, const int
   return VIHMC_OK;
 }
 
-static int dense_run(const vihmc_problem* p, long long C, const float* q, float* logp, float* grad, float* predict_out, void* ws,
-                     size_t ws_bytes, cudaStream_t st) {
+// Log-posterior (out == NULL: logp[C], and grad[C, d] unless grad is NULL) or predict (out != NULL: MLP out[C, N]; DeepONet
+// out[C, N, P] = Bout Tout^T + b0) for C chains, in batches of as many chains as the workspace holds.
+int dense_run(const vihmc_problem* p, long long C, const float* q, float* logp, float* grad, float* out, void* ws, size_t ws_bytes,
+              cudaStream_t st) {
   DensePlan pl;
   if (int rc = make_plan(p, pl)) return rc;
+  const bool predict = out != nullptr;
   if (p->act == VIHMC_ACT_SINE) return fail(VIHMC_ERR_UNSUPPORTED, "dense path implements tanh and relu (the DeepONet reference's set)");
-  if (p->x == nullptr || p->y == nullptr || (pl.deeponet && p->x2 == nullptr)) return fail(VIHMC_ERR_INVALID, "x, x2, y must be device pointers");
+  if (p->x == nullptr || (pl.deeponet && p->x2 == nullptr)) return fail(VIHMC_ERR_INVALID, "x and x2 must be device pointers");
   if ((p->frozen == nullptr) != (p->sens_ind == nullptr)) return fail(VIHMC_ERR_INVALID, "frozen and sens_ind must be given together");
   if (p->sens_ind == nullptr && p->d != p->D) return fail(VIHMC_ERR_INVALID, "d != D requires sens_ind");
-  if (p->prior_scale == 0.0f) return fail(VIHMC_ERR_INVALID, "prior_scale must be non-zero");
+  if (!predict && p->y == nullptr) return fail(VIHMC_ERR_INVALID, "y must be a device pointer");
+  if (!predict && p->prior_scale == 0.0f) return fail(VIHMC_ERR_INVALID, "prior_scale must be non-zero");
   if (ws == nullptr) return fail(VIHMC_ERR_WORKSPACE, "dense path needs a workspace");
   const size_t shared_bytes = (size_t)pl.shared_floats * 4 + 2048;
   if (ws_bytes <= shared_bytes) return fail(VIHMC_ERR_WORKSPACE, "workspace too small");
   const long long cb_max = chains_per_batch(pl, C, ws_bytes - shared_bytes);
   if (cb_max < 1) return fail(VIHMC_ERR_WORKSPACE, "workspace too small for one chain: need %lld bytes", pl.per_chain_floats * 4 + (long long)shared_bytes);
-  const Likelihood lik = make_likelihood(p->loss, p->tau_out);
+  const Likelihood lik = predict ? Likelihood{0.0f, 0.0f, -1.0f} : make_likelihood(p->loss, p->tau_out);
   const long long Dp = pl.Dp, d = p->d, N = pl.N, P = pl.P, Pp = pl.Pp;
   const int wmax = pl.a.max_width() > pl.b.max_width() ? pl.a.max_width() : pl.b.max_width();
 
   SharedBufs sb;
-  if (int rc = prepare_shared(p, pl, ws, predict_out == nullptr, st, sb)) return rc;
+  if (int rc = prepare_shared(p, pl, ws, predict, st, sb)) return rc;
   const float* trunk_in = sb.trunk_in;
-  if (pl.fwd3 && (reinterpret_cast<uintptr_t>(sb.y_pad) & 15u) != 0) return fail(VIHMC_ERR_INVALID, "targets must be 16-byte aligned");
+  if (!predict && pl.fwd3 && (reinterpret_cast<uintptr_t>(sb.y_pad) & 15u) != 0) return fail(VIHMC_ERR_INVALID, "targets must be 16-byte aligned");
 
   for (long long c0 = 0; c0 < C; c0 += cb_max) {
     const int Cb = (int)((C - c0) < cb_max ? (C - c0) : cb_max);
@@ -926,27 +937,27 @@ static int dense_run(const vihmc_problem* p, long long C, const float* q, float*
     for (int l = 0; l < pl.a.n_layers; ++l) acts_a[l] = bb.take((long long)Cb * N * pl.a.dims[l]);
     for (int l = 0; l < pl.b.n_layers; ++l) acts_b[l] = bb.take((long long)Cb * P * pl.b.dims[l]);
     const long long tiles = pl.deeponet ? pl.head_tiles : pl.loss_tiles;
-    float* G = nullptr;
-    if (predict_out == nullptr || !pl.deeponet) G = bb.take((long long)Cb * (pl.deeponet ? N * Pp : N));
+    float* G = bb.take((long long)Cb * (pl.deeponet ? N * Pp : N));
     float* dz0 = bb.take((long long)Cb * pl.R * wmax);
     float* dz1 = bb.take((long long)Cb * pl.R * wmax);
     float* part_ll = bb.take((long long)Cb * tiles);
     float* part_g = bb.take((long long)Cb * tiles);
     float* loglik = bb.take(Cb);
     float* prior_part = bb.take((long long)Cb * ((d + kFinSlab - 1) / kFinSlab));
-    float* scratch = pl.scratch_per_chain > 0 ? bb.take((long long)Cb * pl.scratch_per_chain) : nullptr;
+    const long long scratch_floats = (long long)Cb * pl.scratch_per_chain;
+    float* scratch = scratch_floats > 0 ? bb.take(scratch_floats) : nullptr;
     float* img = pl.img_floats > 0 ? bb.take((long long)Cb * pl.img_floats) : nullptr;
     float* dzs_a[VIHMC_MAX_LAYERS] = {nullptr};
     float* dzs_b[VIHMC_MAX_LAYERS] = {nullptr};
     float* bias_part_a = nullptr;
     float* bias_part_b = nullptr;
-    if (pl.fuse_b && grad != nullptr) {   // the fused backward keeps dz of every layer for the weight gradients
+    if (pl.fuse_b) {   // the fused backward keeps dz of every layer for the weight gradients
       const long long wb = pl.b.max_width();
       for (int l = 0; l < pl.b.n_layers - 1; ++l) dzs_b[l] = bb.take((long long)Cb * P * wb);
       dzs_b[pl.b.n_layers - 1] = dz0;
       bias_part_b = bb.take((long long)Cb * (((P + 127) / 128 + 16) * wb));
     }
-    if (pl.fuse_a && grad != nullptr) {
+    if (pl.fuse_a) {
       const long long wa = pl.a.max_width();
       for (int l = 0; l < pl.a.n_layers - 1; ++l) dzs_a[l] = bb.take((long long)Cb * N * wa);
       dzs_a[pl.a.n_layers - 1] = dz0;
@@ -964,45 +975,35 @@ static int dense_run(const vihmc_problem* p, long long C, const float* q, float*
     const float* qb = q + c0 * d;
 
     if (int rc = scatter_padded(p, pl, sb.pad_map, qb, Wf, Cb, st, c0)) return rc;
-    if (pl.fwd3) {
-      if (int rc = stack_forward3(pl.a, p->x, N, Wf, Dp, acts_a, p->act, Cb, wimg3, ximg_a, xsc_a, st)) return rc;
-      if (int rc = stack_forward3(pl.b, trunk_in, P, Wf, Dp, acts_b, p->act, Cb, wimg3, ximg_b, xsc_b, st)) return rc;
-    } else if (pl.fuse_a) {
-      if (int rc = stack_forward_fused(pl.a, p->x, N, Wf, Dp, acts_a, p->act, Cb, img, st)) return rc;
-    } else {
-      if (int rc = stack_forward(pl.a, p->x, N, Wf, Dp, acts_a, p->act, false, Cb, st)) return rc;
-    }
-    if (pl.deeponet && !pl.fwd3) {
-      if (pl.fuse_b) {
-        if (int rc = stack_forward_fused(pl.b, trunk_in, P, Wf, Dp, acts_b, p->act, Cb, img, st)) return rc;
-      } else {
-        if (int rc = stack_forward(pl.b, trunk_in, P, Wf, Dp, acts_b, p->act, false, Cb, st)) return rc;
-      }
-    }
+    if (int rc = stack_forward_any(pl, pl.a, pl.fuse_a, p->x, N, Wf, acts_a, p->act, Cb, img, wimg3, ximg_a, xsc_a, st)) return rc;
+    if (pl.deeponet)
+      if (int rc = stack_forward_any(pl, pl.b, pl.fuse_b, trunk_in, P, Wf, acts_b, p->act, Cb, img, wimg3, ximg_b, xsc_b, st)) return rc;
 
     if (pl.deeponet) {
-      // head: O = Bout * Tout^T + b0 ; fused residual / loglik partials
+      // head: O = Bout * Tout^T + b0 into out (predict), or G = d loglik / dO with fused loglik partials
       const float* Bout = acts_a[pl.a.n_layers - 1];
       const float* Tout = acts_b[pl.b.n_layers - 1];
       const int K = pl.K;
-      GemmArgs g{};
-      g.A = Bout; g.a_bs = N * K; g.a_sm = K; g.a_sk = 1;
-      g.B = Tout; g.b_bs = P * K; g.b_sk = 1; g.b_sn = K;
-      g.M = (int)N; g.N = (int)P; g.K = K;
-      if (predict_out != nullptr) return fail(VIHMC_ERR_INVALID, "internal: DeepONet predict goes through dense_predict");
-      g.C = G; g.c_bs = N * Pp; g.ldc = Pp; g.row_pad_ok = 1;   // G and the padded targets have Pp floats per row
-      g.bias = Wf; g.bias_bs = Dp;                   // scalar output bias is W[0] (my_make_func.py:52)
-      g.aux = sb.y_pad; g.aux_bs = 0; g.ld_aux = Pp;
-      g.ll_const = lik.ll_const; g.half_prec = lik.half_prec; g.prec = lik.prec;
-      g.part_ll = part_ll; g.part_g = part_g;
+      float* O = predict ? out + c0 * N * P : G;
+      const long long ldo = predict ? P : Pp;   // G and the padded targets have Pp floats per row
       long long parts = tiles;
       if (pl.fwd3) {
         int np = 0;
-        if (int rc = launch_head3(pl, Cb, ximg_a, xsc_a, ximg_b, xsc_b, Wf, Dp, sb.y_pad, Pp, G, N * Pp, Pp, lik, part_ll, part_g, &np, st)) return rc;
+        if (int rc = launch_head3(pl, Cb, ximg_a, xsc_a, ximg_b, xsc_b, Wf, Dp, sb.y_pad, sb.ld_y, O, N * ldo, ldo, lik, part_ll, part_g, &np, st)) return rc;
         parts = np;
       } else {
+        GemmArgs g{};
+        g.A = Bout; g.a_bs = N * K; g.a_sm = K; g.a_sk = 1;
+        g.B = Tout; g.b_bs = P * K; g.b_sk = 1; g.b_sn = K;
+        g.M = (int)N; g.N = (int)P; g.K = K;
+        g.C = O; g.c_bs = N * ldo; g.ldc = ldo; g.row_pad_ok = !predict;
+        g.bias = Wf; g.bias_bs = Dp;                   // scalar output bias is W[0] (my_make_func.py:52)
+        g.aux = sb.y_pad; g.aux_bs = 0; g.ld_aux = sb.ld_y;
+        g.ll_const = lik.ll_const; g.half_prec = lik.half_prec; g.prec = lik.prec;
+        g.part_ll = part_ll; g.part_g = part_g;
         if (int rc = launch_gemm<EPI_HEAD>(g, Cb, st)) return rc;
       }
+      if (predict) continue;
       reduce_partials_kernel<<<(Cb + 3) / 4, 128, 0, st>>>(part_ll, parts, Cb, loglik, 1);
       if (grad != nullptr) {
         reduce_partials_kernel<<<(Cb + 3) / 4, 128, 0, st>>>(part_g, parts, Cb, dWf, Dp);  // d/d b0 = sum G
@@ -1011,37 +1012,36 @@ static int dense_run(const vihmc_problem* p, long long C, const float* q, float*
         h.A = G; h.a_bs = N * Pp; h.a_sm = Pp; h.a_sk = 1;
         h.B = Tout; h.b_bs = P * K; h.b_sk = K; h.b_sn = 1;
         h.C = dz0; h.c_bs = N * K; h.ldc = K; h.M = (int)N; h.N = K; h.K = (int)P;
-        h.kc_hint = 512;   // this product writes 400 KB per slice and chain: 512-deep slices halve that traffic
-                           // (their share of the BASELINE-size gradient error stays below 2e-6, tests/diag_fullsize.py)
-        if (int rc = launch_gemm<EPI_STORE>(h, Cb, st, scratch)) return rc;
+        h.kc_hint = kDBoutChunk;
+        if (int rc = launch_gemm<EPI_STORE>(h, Cb, st, scratch, scratch_floats)) return rc;
         if (bias_part_a != nullptr) {
-          if (int rc = stack_backward_fused(pl.a, p->x, N, Wf, dWf, Dp, acts_a, dzs_a, p->act, Cb, img, bias_part_a, scratch, st)) return rc;
+          if (int rc = stack_backward_fused(pl.a, p->x, N, Wf, dWf, Dp, acts_a, dzs_a, p->act, Cb, img, bias_part_a, scratch, scratch_floats, st)) return rc;
         } else {
-          if (int rc = stack_backward(pl.a, p->x, N, Wf, dWf, Dp, acts_a, dz0, dz1, p->act, Cb, st, scratch)) return rc;
+          if (int rc = stack_backward(pl.a, p->x, N, Wf, dWf, Dp, acts_a, dz0, dz1, p->act, Cb, scratch, scratch_floats, st)) return rc;
         }
         // dTout[p,k] = sum_n G[n,p] Bout[n,k]
         GemmArgs t{};
         t.A = G; t.a_bs = N * Pp; t.a_sm = 1; t.a_sk = Pp;
         t.B = Bout; t.b_bs = N * K; t.b_sk = K; t.b_sn = 1;
         t.C = dz0; t.c_bs = P * K; t.ldc = K; t.M = (int)P; t.N = K; t.K = (int)N;
-        if (int rc = launch_gemm<EPI_STORE>(t, Cb, st, scratch)) return rc;
+        if (int rc = launch_gemm<EPI_STORE>(t, Cb, st, scratch, scratch_floats)) return rc;
         if (bias_part_b != nullptr) {
-          if (int rc = stack_backward_fused(pl.b, trunk_in, P, Wf, dWf, Dp, acts_b, dzs_b, p->act, Cb, img, bias_part_b, scratch, st)) return rc;
+          if (int rc = stack_backward_fused(pl.b, trunk_in, P, Wf, dWf, Dp, acts_b, dzs_b, p->act, Cb, img, bias_part_b, scratch, scratch_floats, st)) return rc;
         } else {
-          if (int rc = stack_backward(pl.b, trunk_in, P, Wf, dWf, Dp, acts_b, dz0, dz1, p->act, Cb, st, scratch)) return rc;
+          if (int rc = stack_backward(pl.b, trunk_in, P, Wf, dWf, Dp, acts_b, dz0, dz1, p->act, Cb, scratch, scratch_floats, st)) return rc;
         }
       }
     } else {
       const float* O = acts_a[pl.a.n_layers - 1];
-      if (predict_out != nullptr) {
-        VIHMC_CUDA_OK(cudaMemcpyAsync(predict_out + c0 * N, O, sizeof(float) * Cb * N, cudaMemcpyDeviceToDevice, st));
+      if (predict) {
+        VIHMC_CUDA_OK(cudaMemcpyAsync(out + c0 * N, O, sizeof(float) * Cb * N, cudaMemcpyDeviceToDevice, st));
         continue;
       }
       mlp_loss_kernel<<<dim3((unsigned)pl.loss_tiles, Cb), 256, 0, st>>>(O, p->y, N, lik.ll_const, lik.half_prec, lik.prec, dz0, part_ll);
       VIHMC_LAUNCH_OK("mlp_loss_kernel");
       reduce_partials_kernel<<<(Cb + 3) / 4, 128, 0, st>>>(part_ll, tiles, Cb, loglik, 1);
       if (grad != nullptr)
-        if (int rc = stack_backward(pl.a, p->x, N, Wf, dWf, Dp, acts_a, dz0, dz1, p->act, Cb, st, scratch)) return rc;
+        if (int rc = stack_backward(pl.a, p->x, N, Wf, dWf, Dp, acts_a, dz0, dz1, p->act, Cb, scratch, scratch_floats, st)) return rc;
     }
     const int slabs = (int)((d + kFinSlab - 1) / kFinSlab);
     finalize_kernel<<<dim3(slabs, Cb), 256, 0, st>>>(dWf, reinterpret_cast<const long long*>(p->sens_ind), qb, p->prior_mu,
@@ -1064,7 +1064,9 @@ int dense_gemm(const float* A, long long a_bs, long long a_sm, long long a_sk, c
   g.A = A; g.a_bs = a_bs; g.a_sm = a_sm; g.a_sk = a_sk;
   g.B = B; g.b_bs = b_bs; g.b_sk = b_sk; g.b_sn = b_sn;
   g.C = C; g.c_bs = c_bs; g.ldc = ldc; g.M = M; g.N = N; g.K = K;
-  return launch_gemm<EPI_STORE>(g, batch, st, scratch, use_tc ? 1 : 0);
+  // the splitk_scratch contract of vihmc_gemm_batched: ceil(K/256) * batch * M * N floats
+  const long long scratch_floats = scratch != nullptr ? (long long)((K + kSplitKChunk - 1) / kSplitKChunk) * batch * M * N : 0;
+  return launch_gemm<EPI_STORE>(g, batch, st, scratch, scratch_floats, use_tc ? 1 : 0);
 }
 
 // vihmc_debug_umma (include/vihmc.h): layout probe of one tcgen05.mma
@@ -1115,78 +1117,6 @@ int dense_xgemm_debug(const float* A, long long lda, const float* B, long long l
   VIHMC_CUDA_OK(cudaFuncSetAttribute(xg::xgemm_test_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, xg::XT_SMEM));
   xg::xgemm_test_kernel<<<dim3(nt, mt, batch), 256, xg::XT_SMEM, st>>>(a_img, a_sc, b_img, b_sc, M, N, K, C, ldc);
   VIHMC_LAUNCH_OK("xgemm_test_kernel");
-  return VIHMC_OK;
-}
-
-int dense_logp_grad(const vihmc_problem* p, long long C, const float* q, float* logp, float* grad, void* ws, size_t ws_bytes,
-                    cudaStream_t st) {
-  return dense_run(p, C, q, logp, grad, nullptr, ws, ws_bytes, st);
-}
-
-// forward only: MLP out[C,N]; DeepONet out[C,N,P] = Bout Tout^T + b0 written straight into `out`
-int dense_predict(const vihmc_problem* p, long long C, const float* q, float* out, void* ws, size_t ws_bytes, cudaStream_t st) {
-  DensePlan pl;
-  if (int rc = make_plan(p, pl)) return rc;
-  if (!pl.deeponet) return dense_run(p, C, q, nullptr, nullptr, out, ws, ws_bytes, st);
-  if (p->act == VIHMC_ACT_SINE) return fail(VIHMC_ERR_UNSUPPORTED, "dense path implements tanh and relu");
-  if (ws == nullptr) return fail(VIHMC_ERR_WORKSPACE, "dense path needs a workspace");
-  const size_t shared_bytes = (size_t)pl.shared_floats * 4 + 2048;
-  if (ws_bytes <= shared_bytes) return fail(VIHMC_ERR_WORKSPACE, "workspace too small");
-  const long long cb_max = chains_per_batch(pl, C, ws_bytes - shared_bytes);
-  if (cb_max < 1) return fail(VIHMC_ERR_WORKSPACE, "workspace too small for one chain");
-  const long long Dp = pl.Dp, d = p->d, N = pl.N, P = pl.P;
-  SharedBufs sb;
-  if (int rc = prepare_shared(p, pl, ws, false, st, sb)) return rc;
-  for (long long c0 = 0; c0 < C; c0 += cb_max) {
-    const int Cb = (int)((C - c0) < cb_max ? (C - c0) : cb_max);
-    Bump bb(sb.batch_base);
-    float* Wf = bb.take((long long)Cb * Dp);
-    bb.take((long long)Cb * Dp);
-    float* acts_a[VIHMC_MAX_LAYERS];
-    float* acts_b[VIHMC_MAX_LAYERS];
-    for (int l = 0; l < pl.a.n_layers; ++l) acts_a[l] = bb.take((long long)Cb * N * pl.a.dims[l]);
-    for (int l = 0; l < pl.b.n_layers; ++l) acts_b[l] = bb.take((long long)Cb * P * pl.b.dims[l]);
-    float* part = bb.take(2LL * Cb * pl.head_tiles);
-    float* img = pl.img_floats > 0 ? bb.take((long long)Cb * pl.img_floats) : nullptr;
-    if (int rc = scatter_padded(p, pl, sb.pad_map, q + c0 * d, Wf, Cb, st, c0)) return rc;
-    if (pl.fwd3) {   // exact-accumulation forward: stacks, then the head kernel in predict mode writes out[c, n, p] directly
-      unsigned char* wimg3 = reinterpret_cast<unsigned char*>(bb.take((long long)Cb * pl.wimg3_floats));
-      unsigned char* ximg_a = reinterpret_cast<unsigned char*>(bb.take((long long)Cb * pl.ximg_a_floats));
-      unsigned char* ximg_b = reinterpret_cast<unsigned char*>(bb.take((long long)Cb * pl.ximg_b_floats));
-      float* xsc_a = bb.take((long long)Cb * pl.m_tiles * 128);
-      float* xsc_b = bb.take((long long)Cb * pl.p_tiles128 * 128);
-      if (int rc = stack_forward3(pl.a, p->x, N, Wf, Dp, acts_a, p->act, Cb, wimg3, ximg_a, xsc_a, st)) return rc;
-      if (int rc = stack_forward3(pl.b, sb.trunk_in, P, Wf, Dp, acts_b, p->act, Cb, wimg3, ximg_b, xsc_b, st)) return rc;
-      Likelihood none{};
-      if (int rc = launch_head3(pl, Cb, ximg_a, xsc_a, ximg_b, xsc_b, Wf, Dp, nullptr, 0, out + c0 * N * P, N * P, P, none, part,
-                                part + (long long)Cb * pl.head_tiles, nullptr, st)) return rc;
-      continue;
-    }
-    if (pl.fuse_a) {
-      if (int rc = stack_forward_fused(pl.a, p->x, N, Wf, Dp, acts_a, p->act, Cb, img, st)) return rc;
-    } else {
-      if (int rc = stack_forward(pl.a, p->x, N, Wf, Dp, acts_a, p->act, false, Cb, st)) return rc;
-    }
-    if (pl.fuse_b) {
-      if (int rc = stack_forward_fused(pl.b, sb.trunk_in, P, Wf, Dp, acts_b, p->act, Cb, img, st)) return rc;
-    } else {
-      if (int rc = stack_forward(pl.b, sb.trunk_in, P, Wf, Dp, acts_b, p->act, false, Cb, st)) return rc;
-    }
-    // O = Bout Tout^T + b0 through the HEAD epilogue with a zero target and prec = -1: C = -(-1) * (O - 0) = O
-    GemmArgs g{};
-    const int K = pl.K;
-    g.A = acts_a[pl.a.n_layers - 1]; g.a_bs = N * K; g.a_sm = K; g.a_sk = 1;
-    g.B = acts_b[pl.b.n_layers - 1]; g.b_bs = P * K; g.b_sk = 1; g.b_sn = K;
-    g.M = (int)N; g.N = (int)P; g.K = K;
-    g.C = out + c0 * N * P; g.c_bs = N * P; g.ldc = P;
-    g.bias = Wf; g.bias_bs = Dp;
-    g.part_ll = part; g.part_g = part + (long long)Cb * pl.head_tiles;
-    g.prec = -1.0f;
-    float* zero_row = bb.take(pl.Pp);   // target row of zeros shared by every output row (ld_aux = 0)
-    VIHMC_CUDA_OK(cudaMemsetAsync(zero_row, 0, sizeof(float) * pl.Pp, st));
-    g.aux = zero_row; g.aux_bs = 0; g.ld_aux = 0;
-    if (int rc = launch_gemm<EPI_HEAD>(g, Cb, st)) return rc;
-  }
   return VIHMC_OK;
 }
 

@@ -53,7 +53,7 @@ struct GemmArgs {
   // split-K (EPI_STORE only): blockIdx.z = b * splits + s handles k in [s*kc, min(K,(s+1)*kc)) and writes its
   // partial product to split_buf[(s*batch + b), M, N]; splits <= 1 means a plain GEMM
   int splits, kc, batch;
-  int kc_hint;   // host side: preferred split-K slice length for this product (0: the default, splitk_chunk())
+  int kc_hint;   // host side: preferred split-K slice length for this product (0: the default, kSplitKChunk)
   int slice_tiles;   // TMEM-A kernels: k-tiles per accumulation chain; the CTA sums its slices itself (0: one chain per CTA)
   float* split_buf;
   // row sums of opA over this CTA's K range (EPI_STORE, A staged MN-major, N <= 128): rowsum_part[(s*batch + b), M].
@@ -886,26 +886,17 @@ __global__ void rowsum_finish_kernel(const float* __restrict__ part, int splits,
 // The fp32 accumulate of tcgen05.mma truncates toward zero: a chain of k accumulations shrinks the sum by ~k/2 ulp.  At BASELINE
 // size (K = 10201) 1152-deep slices left 1.3e-5 relative error on the trunk's weight gradients (tests/diag_fullsize.py); with
 // 256-deep slices (32 chained accumulations) summed by round-to-nearest adds it is below 4e-6.
-// VIHMC_SPLITK_CHUNK overrides the slice length (A/B runs of accuracy against time).
-inline int splitk_chunk() {
-  static const int v = []() {
-    const char* e = getenv("VIHMC_SPLITK_CHUNK");
-    const int c = e != nullptr ? atoi(e) : 0;
-    return c >= 64 ? c / 16 * 16 : 256;
-  }();
-  return v;
-}
-#define kSplitKChunk (::vihmc::splitk_chunk())          /* K slice per CTA once K exceeds kSplitKThreshold */
-#define kSplitKThreshold (::vihmc::splitk_chunk() + ::vihmc::splitk_chunk() / 2)   /* K = 500 (the M = 2 split closures) -> two slices */
-
+constexpr int kSplitKChunk = 256;       // K slice per CTA once K exceeds 1.5 slices (K = 500, the M = 2 split closures -> two slices)
 constexpr int kFillSplitMinK = 512;     // medium reductions are split only to put more CTAs on the GPU (few chains)
 constexpr int kFillSplitMax = 8;
 
-// floats of scratch a split-K GEMM of this shape needs (0 if it will not be split)
-inline long long splitk_scratch_floats(int M, int N, int K, int batch) {
-  if (K > kSplitKThreshold) return (long long)((K + kSplitKChunk - 1) / kSplitKChunk) * batch * M * N;
-  if (K >= kFillSplitMinK) return (long long)kFillSplitMax * batch * M * N;
-  return 0;
+// The most K slices splitk_plan can choose for a reduction of K with this slice hint, at any batch: a split product needs
+// slices * batch * M * N floats of scratch.
+inline int splitk_max_slices(int K, int kc_hint) {
+  const int chunk = kc_hint > 0 ? kc_hint : kSplitKChunk;
+  if (K > chunk + chunk / 2) return (K + chunk - 1) / chunk;
+  if (K >= kFillSplitMinK) return K / 128 < kFillSplitMax ? K / 128 : kFillSplitMax;
+  return 1;
 }
 
 // shapes the tensor-core kernel is used for; everything else stays on the FP32-SIMT kernel
@@ -929,36 +920,21 @@ inline int operand_mode(const float* base, long long bs, long long s_r, long lon
   return tc::LOAD_SCALAR;
 }
 
-// rowsum_out (EPI_STORE, optional): receives sum_k opA[b][m, k] at rowsum_out[b*rowsum_bs + m]; rowsum_part is scratch of
-// ceil(K/1024) * batch * M floats.  Returns VIHMC_ERR_UNSUPPORTED-free: when the fused row sums cannot be used
-// (*rowsum_done stays 0) the caller computes them itself.
-template <int EPI>
-static int launch_tc_gemm(GemmArgs g, int batch, cudaStream_t st, float* scratch = nullptr, float* rowsum_part = nullptr,
-                          float* rowsum_out = nullptr, long long rowsum_bs = 0, int* rowsum_done = nullptr) {
-  const int a_mode = operand_mode(g.A, g.a_bs, g.a_sm, g.a_sk);
-  const int b_mode = operand_mode(g.B, g.b_bs, g.b_sn, g.b_sk);
-  auto k = tc::tc_gemm_kernel<EPI>;
-  static bool configured = false;
-  if (!configured) {
-    VIHMC_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
-    configured = true;
-  }
-  // TMEM-A variant: plain-store products with one n-tile of at most 112 columns and a vector-staged B (the weight-gradient
-  // GEMMs and the two head-backward products).  VIHMC_TC_TMEMA=0 keeps the shared-memory A path.
-  static const bool atm_on = []() { const char* e = getenv("VIHMC_TC_TMEMA"); return e == nullptr || atoi(e) != 0; }();
-  const bool use_atm = EPI == EPI_STORE && atm_on && g.N <= tc::ATM_ACCN;
+// Sets g.splits, g.kc and g.slice_tiles for `batch` products.  Only EPI_STORE products split, and only when scratch for the
+// partial products is available (can_split); use_atm selects the TMEM-A kernel.  g.splits never exceeds
+// splitk_max_slices(g.K, g.kc_hint).
+inline void splitk_plan(GemmArgs& g, int batch, bool use_atm, bool can_split) {
   g.splits = 1;
   g.batch = batch;
   const int chunk = g.kc_hint > 0 ? g.kc_hint : kSplitKChunk, thresh = chunk + chunk / 2;
-  // VIHMC_TC_INSLICE=0: one accumulation chain per CTA as in the first round-2 version (A/B runs)
-  static const bool inslice = []() { const char* e = getenv("VIHMC_TC_INSLICE"); return e == nullptr || atoi(e) != 0; }();
-  g.slice_tiles = (use_atm && inslice) ? chunk / tc::BK : 0;
-  if (use_atm && inslice && scratch != nullptr && g.K > thresh) {
+  const int max_splits = splitk_max_slices(g.K, g.kc_hint);
+  g.slice_tiles = use_atm ? chunk / tc::BK : 0;
+  if (!can_split) return;
+  const long long slots = 2LL * tc_num_sms();
+  if (use_atm && g.K > thresh) {
     // TMEM-A kernels sum their slices in shared memory: cross-CTA splits only fill the GPU.  Cost of a choice in k-units per
     // CTA slot: rounds x (slice-aligned K range + the partial tile's write and read, ~106 k-units of operand traffic)
     const long long tiles = (long long)((g.M + tc::BM - 1) / tc::BM) * batch;
-    const int max_splits = (g.K + chunk - 1) / chunk;
-    const long long slots = 2LL * tc_num_sms();
     long long best_cost = -1;
     for (int sp = 1; sp <= max_splits; ++sp) {
       const int kc = ((g.K + sp - 1) / sp + chunk - 1) / chunk * chunk;
@@ -968,17 +944,14 @@ static int launch_tc_gemm(GemmArgs g, int batch, cudaStream_t st, float* scratch
       if (best_cost < 0 || cost < best_cost) { best_cost = cost; g.kc = kc; }
     }
     g.splits = (g.K + g.kc - 1) / g.kc;
-    g.split_buf = scratch;
-    if ((long long)batch * g.splits > 65535) return fail(VIHMC_ERR_UNSUPPORTED, "gemm: batch * splits > 65535");
-  } else if (EPI == EPI_STORE && scratch != nullptr && g.K > thresh) {
+  } else if (g.K > thresh) {
     // long reductions (dW = dZ^T X over thousands of rows): bound the length of one TMEM accumulation chain
     // (its fp32 accumulate truncates) and sum the slices with round-to-nearest adds
-    // Slice length between 1024 (what the scratch is sized for) and 2048 (the accuracy bound), chosen so that the CTAs
+    // Slice length between one chunk (what the scratch is sized for) and 1.5 chunks, chosen so that the CTAs
     // fill whole rounds of the GPU: 2 CTAs per SM hold TMEM at a time, and e.g. 64 chains x 10 slices = 640 CTAs would
     // run 3 rounds for 2.16 rounds of work where 9 slices of 1152 run 2.
     const long long tiles = (long long)((g.N + tc::BN - 1) / tc::BN) * ((g.M + tc::BM - 1) / tc::BM) * batch;
-    const int max_splits = (g.K + chunk - 1) / chunk, min_splits = (g.K + thresh - 1) / thresh;
-    const long long slots = 2LL * tc_num_sms();
+    const int min_splits = (g.K + thresh - 1) / thresh;
     long long best_cost = -1;
     for (int sp = max_splits; sp >= min_splits && sp >= 1; --sp) {
       const int kc = ((g.K + sp - 1) / sp + tc::BK - 1) / tc::BK * tc::BK;
@@ -987,19 +960,44 @@ static int launch_tc_gemm(GemmArgs g, int batch, cudaStream_t st, float* scratch
       if (best_cost < 0 || cost < best_cost) { best_cost = cost; g.kc = kc; }
     }
     g.splits = (g.K + g.kc - 1) / g.kc;
-    g.split_buf = scratch;
-    if ((long long)batch * g.splits > 65535) return fail(VIHMC_ERR_UNSUPPORTED, "gemm: batch * splits > 65535");
-  } else if (EPI == EPI_STORE && scratch != nullptr && g.K >= kFillSplitMinK) {
+  } else if (g.K >= kFillSplitMinK) {
     // medium reduction, few output tiles (the branch's weight gradients: 64 chains = 64 CTAs): split to fill the GPU
     const long long tiles = (long long)((g.N + tc::BN - 1) / tc::BN) * ((g.M + tc::BM - 1) / tc::BM) * batch;
-    long long sp = 2LL * tc_num_sms() / tiles;
-    if (sp > kFillSplitMax) sp = kFillSplitMax;
-    if (sp > g.K / 128) sp = g.K / 128;
+    long long sp = slots / tiles;
+    if (sp > max_splits) sp = max_splits;
     if (sp >= 2 && (long long)batch * sp <= 65535) {
       g.kc = (int)(((g.K + sp - 1) / sp + tc::BK - 1) / tc::BK * tc::BK);
       g.splits = (g.K + g.kc - 1) / g.kc;
-      g.split_buf = scratch;
     }
+  }
+}
+
+// scratch: room for scratch_floats floats of split-K partial products (splitk_max_slices(K, kc_hint) * batch * M * N are
+// always enough); VIHMC_ERR_WORKSPACE if the plan needs more.
+// rowsum_out (EPI_STORE, optional): receives sum_k opA[b][m, k] at rowsum_out[b*rowsum_bs + m]; rowsum_part is scratch of
+// splits * batch * M floats (at most splitk_max_slices(K, kc_hint) * batch * M).  When the fused row sums cannot be used
+// (*rowsum_done stays 0) the caller computes them itself.
+template <int EPI>
+static int launch_tc_gemm(GemmArgs g, int batch, cudaStream_t st, float* scratch = nullptr, long long scratch_floats = 0,
+                          float* rowsum_part = nullptr, float* rowsum_out = nullptr, long long rowsum_bs = 0, int* rowsum_done = nullptr) {
+  const int a_mode = operand_mode(g.A, g.a_bs, g.a_sm, g.a_sk);
+  const int b_mode = operand_mode(g.B, g.b_bs, g.b_sn, g.b_sk);
+  auto k = tc::tc_gemm_kernel<EPI>;
+  static bool configured = false;
+  if (!configured) {
+    VIHMC_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+    configured = true;
+  }
+  // TMEM-A variant: plain-store products with one n-tile of at most 112 columns (the weight-gradient GEMMs and the two
+  // head-backward products)
+  const bool use_atm = EPI == EPI_STORE && g.N <= tc::ATM_ACCN;
+  splitk_plan(g, batch, use_atm, EPI == EPI_STORE && scratch != nullptr);
+  if (g.splits > 1) {
+    if ((long long)batch * g.splits > 65535) return fail(VIHMC_ERR_UNSUPPORTED, "gemm: batch * splits > 65535");
+    if ((long long)g.splits * batch * g.M * g.N > scratch_floats)
+      return fail(VIHMC_ERR_WORKSPACE, "gemm: %d K slices need %lld floats of scratch, %lld given", g.splits,
+                  (long long)g.splits * batch * g.M * g.N, scratch_floats);
+    g.split_buf = scratch;
   }
   const int tiles_n = (g.N + tc::BN - 1) / tc::BN, tiles_m = (g.M + tc::BM - 1) / tc::BM;
   const bool fuse_rowsum = EPI == EPI_STORE && rowsum_part != nullptr && rowsum_out != nullptr && (a_mode == tc::LOAD_MNVEC || use_atm);

@@ -164,7 +164,7 @@ def gemm_batched(A: torch.Tensor, B: torch.Tensor, tensor_cores: bool = True) ->
     out = torch.empty(batch, M, N, dtype=torch.float32, device=dev)
     scratch = None
     if tensor_cores and K > 2048:
-        scratch = torch.empty(((K + 1023) // 1024) * batch * M * N, dtype=torch.float32, device=dev)
+        scratch = torch.empty(((K + 255) // 256) * batch * M * N, dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
         _lib.check(_lib.load().vihmc_gemm_batched(A.data_ptr(), A.stride(0), A.stride(1), A.stride(2), B.data_ptr(), B.stride(0),
                                                   B.stride(1), B.stride(2), out.data_ptr(), M * N, N, M, N, K, batch,
