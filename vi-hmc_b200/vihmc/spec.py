@@ -198,6 +198,12 @@ class LogProbSpec:
                 raise ValueError("DeepONet spec needs trunk coordinates x2")
             if tuple(self.y.shape) != (self.N, int(self.x2.shape[0])):
                 raise ValueError("y must be [N, P]")
+            # the kernels read x2 with a fixed row stride (2 for the (t, x) pairs of the feature layer, in_trunk for raw
+            # trunk inputs): any other width would be read as the wrong numbers, not refused
+            cols = 2 if self.arch.impose_bc else self.arch.in_trunk
+            if self.x2.dim() != 2 or int(self.x2.shape[1]) != cols:
+                what = "(t, x) pairs for the feature layer" if self.arch.impose_bc else f"in_trunk = {cols} raw trunk inputs"
+                raise ValueError(f"x2 must be [P, {cols}] ({what}), got {tuple(self.x2.shape)}")
         loss_code(self.loss)
         if self.trunk_subsample is not None:
             if self.model_kind != MODEL_DEEPONET:
