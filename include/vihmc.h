@@ -258,7 +258,10 @@ VIHMC_API int vihmc_mlp_sensitivity(const vihmc_problem* prob, const float* weig
  * over the prob->N validation functions prob->x [N, in_a] and the prob->P trunk points prob->x2 they share.  The Jacobian
  * (N * P * D floats in the reference) is never formed: the sum over p (over n for trunk parameters) is folded into a K x K
  * Gram matrix whose Cholesky rows seed K back-propagations per row (csrc/don_sensitivity.cu).  d == D, frozen / sens_ind
- * NULL, tanh or relu, widths and output neurons <= 128; y, prior and likelihood fields are not used.
+ * NULL, tanh or relu, widths and output neurons <= 128, branch and raw trunk inputs (in_a, in_b) <= 29 056 (the forward
+ * kernel holds two rows of max(input, widths) floats in a block's 227 KB of shared memory); y, prior and likelihood fields
+ * are not used.  An unsupported architecture is refused with VIHMC_ERR_UNSUPPORTED and its reason before any pointer is
+ * read, and vihmc_deeponet_sensitivity_workspace_bytes returns 0 for it.
  */
 VIHMC_API size_t vihmc_deeponet_sensitivity_workspace_bytes(const vihmc_problem* prob);
 VIHMC_API int vihmc_deeponet_sensitivity(const vihmc_problem* prob, const float* weights, const float* sigma, float* scores,

@@ -24,6 +24,9 @@ namespace vihmc {
 namespace {
 
 constexpr int kMaxDim = 128;   // widths, output neurons <= 128 (backward tile buffers live in shared memory)
+// the forward kernel keeps two rows of max(input, widths) floats in shared memory: 227 KB, the most a block may opt in to,
+// bounds the inputs at 29 056
+constexpr size_t kMaxForwardSmem = 232448;
 
 struct StackDesc {
   int n_layers, in_dim, maxdim;
@@ -227,6 +230,7 @@ inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 struct Plan {
   StackDesc br, tr;
   int K, NB;
+  size_t fwd_smem;
   size_t off_feat, off_acts_br, off_acts_tr, off_E_br, off_E_tr, off_G, off_R, total;
 };
 
@@ -262,6 +266,10 @@ int make_plan(const vihmc_problem* p, Plan& pl) {
   for (int l = 0; l < p->n_layers_b; ++l) maxw = p->dims_b[l] > maxw ? p->dims_b[l] : maxw;
   if (maxw > kMaxDim) return fail(VIHMC_ERR_UNSUPPORTED, "deeponet sensitivity: widths up to %d are implemented (got %d)", kMaxDim, maxw);
   pl.NB = (maxw + 15) / 16;
+  pl.fwd_smem = (size_t)2 * (pl.br.maxdim > pl.tr.maxdim ? pl.br.maxdim : pl.tr.maxdim) * sizeof(float);
+  if (pl.fwd_smem > kMaxForwardSmem)
+    return fail(VIHMC_ERR_UNSUPPORTED, "deeponet sensitivity: branch / trunk inputs up to %d are implemented (got %d / %d)",
+                (int)(kMaxForwardSmem / (2 * sizeof(float))), p->in_a, p->in_b);
   size_t o = 0;
   pl.off_feat = o;    o += align256((size_t)p->P * 5 * sizeof(float));
   pl.off_acts_br = o; o += align256((size_t)acts_br * sizeof(float));
@@ -318,7 +326,8 @@ int run(const vihmc_problem* p, const Plan& pl, const float* w, const float* sig
     VIHMC_LAUNCH_OK("don_sens_features_kernel");
     trunk_in = feat;
   }
-  // 1. activations at the VI means
+  // 1. activations at the VI means (inputs past 6 144 floats need more than the 48 KB of shared memory a launch gets by default)
+  VIHMC_CUDA_OK(cudaFuncSetAttribute(don_sens_forward_kernel<ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.fwd_smem));
   don_sens_forward_kernel<ACT><<<(unsigned)p->N, 128, 2 * pl.br.maxdim * sizeof(float), st>>>(pl.br, w, p->x, p->in_a, acts_br);
   VIHMC_LAUNCH_OK("don_sens_forward_kernel(branch)");
   don_sens_forward_kernel<ACT><<<(unsigned)p->P, 128, 2 * pl.tr.maxdim * sizeof(float), st>>>(pl.tr, w, trunk_in, p->in_b, acts_tr);
@@ -368,10 +377,11 @@ int deeponet_sensitivity(const vihmc_problem* prob, const float* weights, const 
                          cudaStream_t st) {
   if (prob->d != prob->D || prob->sens_ind != nullptr || prob->frozen != nullptr)
     return fail(VIHMC_ERR_INVALID, "deeponet sensitivity: pass the full weight vector (d == D, no frozen / sens_ind)");
-  if (weights == nullptr || sigma == nullptr || scores == nullptr || prob->x == nullptr || prob->x2 == nullptr)
-    return fail(VIHMC_ERR_INVALID, "deeponet sensitivity: null pointer");
+  // the plan first: an unsupported architecture is reported with its reason even when called with NULL buffers
   Plan pl{};
   if (int rc = make_plan(prob, pl)) return rc;
+  if (weights == nullptr || sigma == nullptr || scores == nullptr || prob->x == nullptr || prob->x2 == nullptr)
+    return fail(VIHMC_ERR_INVALID, "deeponet sensitivity: null pointer");
   if (ws == nullptr || ws_bytes < pl.total)
     return fail(VIHMC_ERR_WORKSPACE, "deeponet sensitivity: workspace too small, need %zu bytes", pl.total);
   char* base = static_cast<char*>(ws);
